@@ -11,11 +11,18 @@ independent, no data-path collective; the per-rank digest tables are all-gathere
             input -> parallel_map.InputPumper, against a null control plane / object store
   e2e_pinned  the same payloads through batch.hash_table_host on page-locked host memory (round 1's e2e figure)
   roofline  lane_hash_kernel: algorithmic bytes / measured kernel time vs the measured HBM copy peak
-  cpu_baseline  the reference's own get_upload_hashes (unmodified hash_utils.py from baseline/_ref through
-            oracle/ref_shim.py; oracle/ref_port.py only if that copy is missing) on the host cores, bounded sample
+  cpu_baseline  the reference's own get_upload_hashes (unmodified hash_utils.py from the checkout named by
+            B200H_REFERENCE_ROOT, through oracle/ref_shim.py; oracle/ref_port.py without one) on the host cores,
+            bounded sample
 
+`--steps` timed steps (after `--warmup` untimed ones) are run on every leg above but the CPU baseline.
 `--impl reference` times that same reference implementation (hashlib underneath, all host threads) on the same
 workload shape and prints the same JSON line.
+`--dump-outputs DIR` writes, after the timed steps, the digest tables the last step of each GPU leg returned as
+float32 DIR/<name>.npy (one row per message, one column per digest byte): sha256 / md5 (HBM-resident),
+e2e_pinned_sha256 / e2e_pinned_md5, e2e_sha256 / e2e_md5 (as BlobCreate received them).  The payloads are
+generated from a fixed seed, so two builds can be compared output for output.  Past OUTPUT_DUMP_BYTES in all, a
+fixed, seeded sample of rows is written, with their indices in rows.npy.
 """
 from __future__ import annotations
 
@@ -101,6 +108,29 @@ class ClockSampler:
         return self.summarize(rows, self.proc is not None)
 
 
+OUTPUT_DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir: str, tables: dict) -> None:
+    """``tables``: name -> uint8[n, k] digest table (the same n for all).  Each is written as float32
+    ``out_dir/<name>.npy``; if that would pass OUTPUT_DUMP_BYTES, the same fixed, seeded sample of rows of every
+    table is written instead, and the sampled row indices as float64 ``rows.npy``."""
+    import numpy as np
+
+    n = len(next(iter(tables.values())))
+    row_bytes = sum(4 * t.shape[1] for t in tables.values())
+    budget = OUTPUT_DUMP_BYTES - 4096  # room for the .npy headers
+    rows = None
+    if n * row_bytes > budget:
+        rows = np.sort(np.random.default_rng(0).choice(n, budget // (row_bytes + 8), replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in tables.items():
+        assert len(t) == n, name
+        np.save(os.path.join(out_dir, f"{name}.npy"), (t if rows is None else t[rows]).astype(np.float32))
+    if rows is not None:
+        np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
+
+
 def env_rank():
     return (int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0)))
 
@@ -118,8 +148,8 @@ _REF = None
 
 
 def reference_hasher():
-    """(callable, kind): the reference's OWN ``get_upload_hashes`` (unmodified hash_utils.py from baseline/_ref or
-    /root/reference, loaded through oracle/ref_shim.py) -> kind "reference"; if no copy travelled, the hashlib
+    """(callable, kind): the reference's OWN ``get_upload_hashes`` (unmodified hash_utils.py from the checkout named
+    by B200H_REFERENCE_ROOT, loaded through oracle/ref_shim.py) -> kind "reference"; without one, the hashlib
     port in oracle/ref_port.py -> kind "port".  Both make exactly the same hashlib calls."""
     global _REF
     if _REF is None:
@@ -386,8 +416,8 @@ def run_gpu(args) -> None:
     del data
     torch.cuda.empty_cache()
     off_h = (np.arange(N_MSG, dtype=np.uint64) * np.uint64(MSG_BYTES))
-    e2e_steps = max(1, min(args.steps, 3))
-    e2e_warm = max(1, min(args.warmup, 3))
+    e2e_steps = args.steps
+    e2e_warm = args.warmup
 
     def all_gather_host_table(packed: np.ndarray):
         if world > 1:  # every rank ends the step holding the whole job's digest table
@@ -399,7 +429,7 @@ def run_gpu(args) -> None:
         return tab
 
     for _ in range(e2e_warm):  # warm-up (first call allocates the wave buffers)
-        table = pinned_step()
+        pinned_step()
     barrier()
     t0 = time.perf_counter()
     for _ in range(e2e_steps):
@@ -458,6 +488,9 @@ def run_gpu(args) -> None:
     pump_value = world * total_bytes * e2e_steps / GiB / pump_s
     ptab = requests_table(stub)  # what BlobCreate was told, checked after the timed region
     pump_same = bool(len(ptab) == N_MSG and np.array_equal(ptab[:, :32], sha_dev) and np.array_equal(ptab[:, 32:], md5_dev))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"sha256": sha_dev, "md5": md5_dev, "e2e_pinned_sha256": table.sha256,
+                                         "e2e_pinned_md5": table.md5, "e2e_sha256": ptab[:, :32], "e2e_md5": ptab[:, 32:]})
 
     # ---- CPU baseline (rank 0, N=1): the reference's hashlib path on a bounded sample of the same bytes
     cpu = None
@@ -550,7 +583,10 @@ def main():
     ap.add_argument("--steps", type=int, default=5)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's digest tables as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,8 +1,8 @@
 """oracle/gen_golden.py -- regenerates tests/golden/*.json from the UNMODIFIED reference.
 
-Run in the build container only (needs /root/reference):  ``python -m oracle.gen_golden``
+Needs a source checkout of the original modal client:  ``B200H_REFERENCE_ROOT=<checkout> python -m oracle.gen_golden``
 Inputs are stored as small recipes (modal_client_b200.synth.materialize), outputs are whatever the
-reference's own functions returned.  The GPU box never runs this; it only reads the JSON.
+reference's own functions returned.  The tests only read the JSON, so they need no copy of the reference.
 """
 from __future__ import annotations
 
@@ -341,12 +341,132 @@ def gen_mount_select():
             "tree": {k: list(v) for k, v in MOUNT_TREE.items()}, "cases": cases}
 
 
+# ------------------------------------------------------------------ what the reference's callers see of the seam
+
+
+def _reference_constant(rel, name):
+    """A module constant of the reference read from its source text (modules that need the control plane to import)."""
+    import re
+
+    text = open(os.path.join(os.path.dirname(ref_shim.package_dir()), "modal", rel)).read()
+    m = re.search(rf"^{name}\s*(?::[^=]+)?=\s*\(?\s*([^#\n]+)", text, flags=re.M)
+    return eval(m.group(1).strip().rstrip(")"))  # noqa: S307 - arithmetic literals of the reference
+
+
+def gen_seam(h, b, seg):
+    """What crosses the drop-in seam when the reference's own callers run: the patchable module constants, the
+    get_upload_hashes calls of its spec builder (argument kind, stream position, supplied digests, what came back),
+    the BytesIOSegmentPayload objects its multipart upload builds (segment, chunk size, bytes sent, MD5 checked
+    against the ETag), and its get_upload_hashes / _find_end_of_block on a few more inputs."""
+    import hashlib
+
+    constants = {"hash_utils": {"HASH_CHUNK_SIZE": h.HASH_CHUNK_SIZE},
+                 "blob_utils": {k: getattr(b, k) for k in ["MAX_OBJECT_SIZE_BYTES", "MAX_ASYNC_OBJECT_SIZE_BYTES",
+                                                           "LARGE_FILE_LIMIT", "BLOB_MAX_PARALLELISM",
+                                                           "DEFAULT_SEGMENT_CHUNK_SIZE", "MULTIPART_UPLOAD_THRESHOLD",
+                                                           "BLOCK_SIZE"]}}
+    for rel, name in [("mount.py", "MOUNT_PUT_FILE_CLIENT_TIMEOUT"), ("volume.py", "VOLUME_PUT_FILE_CLIENT_TIMEOUT"),
+                      ("network_file_system.py", "NETWORK_FILE_SYSTEM_PUT_FILE_CLIENT_TIMEOUT"),
+                      ("parallel_map.py", "MAP_INVOCATION_CHUNK_SIZE"),
+                      ("parallel_map.py", "SPAWN_MAP_INVOCATION_CHUNK_SIZE")]:
+        constants.setdefault(rel[:-3], {})[name] = _reference_constant(rel, name)
+
+    # the spec builder's calls into hash_utils, one list per tests/golden/file_specs.json case
+    spec_calls = []
+    real = b.get_upload_hashes
+
+    def recording(data, **kw):
+        is_stream = not isinstance(data, (bytes, bytearray, memoryview))
+        call = {"stream": is_stream, "pos": data.tell() if is_stream else None, "kwargs": kw}
+        up = real(data, **kw)
+        call.update(pos_after=data.tell() if is_stream else None, sha256_hex=up.sha256_hex(), md5_hex=up.md5_hex())
+        spec_calls[-1].append(call)
+        return up
+
+    b.get_upload_hashes = recording
+    try:
+        for c in json.load(open(os.path.join(OUT, "file_specs.json")))["cases"]:
+            saved = {k: getattr(b, k) for k in c["patch"]}
+            spec_calls.append([])
+            try:
+                for k, v in c["patch"].items():
+                    setattr(b, k, v)
+                b.get_file_upload_spec_from_fileobj(io.BytesIO(materialize(c["input"])), PurePosixPath(c["mount_filename"]),
+                                                    0o100644 if not c["patch"] else 0o755)
+            finally:
+                for k, v in saved.items():
+                    setattr(b, k, v)
+    finally:
+        b.get_upload_hashes = real
+
+    # the multipart upload's segment payloads (the reference checks each one's MD5 against the part's ETag)
+    payloads = []
+
+    class RecordingPayload(seg.BytesIOSegmentPayload):
+        def __init__(self, bytes_io, segment_start, segment_length, chunk_size, progress_report_cb=None):
+            super().__init__(bytes_io, segment_start, segment_length, chunk_size, progress_report_cb)
+            payloads.append({"initial_pos": self.initial_seek_pos, "segment_start": segment_start,
+                             "segment_length": segment_length, "chunk_size": chunk_size})
+
+    part_etags = {}
+
+    async def put(upload_url, payload, content_md5_b64=None, content_type=None):
+        sink = _Sink()
+        with payload.reset_on_error():  # which resets the payload on the way out, as in blob_utils.py:118
+            await payload.write(sink)
+            body = b"".join(sink.chunks)
+            part_etags[int(upload_url)] = hashlib.md5(body).digest()  # what S3 answers: the MD5 of the body it got
+            local = payload.md5_checksum().hexdigest()
+            assert local == part_etags[int(upload_url)].hex()  # the check at blob_utils.py:150-152
+        payloads[int(upload_url)].update(sent_sha256=hashlib.sha256(body).hexdigest(), md5_hex=local)
+        return local
+
+    class Session:
+        async def post(self, url, data=None, skip_auto_headers=None):
+            joined = b"".join(part_etags[i] for i in sorted(part_etags))
+            etag = f"{hashlib.md5(joined).hexdigest()}-{len(part_etags)}"
+
+            class Resp:
+                status = 200
+
+                async def text(self):
+                    return f'<ETag>"{etag}"</ETag>'
+            return Resp()
+
+    class Reg:
+        get_session = staticmethod(Session)
+
+    mp_input, part_len, chunk = synth(77, 10 * 1000 + 123), 1000, 256
+    data = materialize(mp_input)
+    saved = b._upload_to_s3_url, b.ClientSessionRegistry, seg.BytesIOSegmentPayload
+    b._upload_to_s3_url, b.ClientSessionRegistry, seg.BytesIOSegmentPayload = put, Reg, RecordingPayload
+    try:
+        asyncio.run(b.perform_multipart_upload(io.BytesIO(data), content_length=len(data), max_part_size=part_len,
+                                               part_urls=[str(i) for i in range(11)], completion_url="done",
+                                               upload_chunk_size=chunk))
+    finally:
+        b._upload_to_s3_url, b.ClientSessionRegistry, seg.BytesIOSegmentPayload = saved
+
+    upload_hashes = []
+    for seed, n in [(900, 0), (901, 1), (902, 70001), (903, 300000)]:
+        r = synth(seed, n)
+        d = materialize(r)
+        up = h.get_upload_hashes(io.BytesIO(d))
+        upload_hashes.append({"input": r, "md5_base64": up.md5_base64, "sha256_base64": up.sha256_base64,
+                              "end_of_block_with_9_zeros": b._find_end_of_block(lambda: io.BytesIO(d + bytes(9)), 0, n + 9)})
+    return {"source": "py/modal/_utils/{hash_utils,blob_utils,bytes_io_segment_payload}.py and the constants of "
+                      "mount.py / volume.py / network_file_system.py / parallel_map.py (unmodified, executed or read)",
+            "constants": constants, "spec_builder_calls": spec_calls,
+            "multipart": {"input": mp_input, "part_len": part_len, "chunk": chunk, "payloads": payloads},
+            "upload_hashes": upload_hashes}
+
+
 def main():
     h, b, seg = ref_shim.load()
     os.makedirs(OUT, exist_ok=True)
     for name, doc in [("hash_utils.json", gen_hash_utils(h)), ("file_specs.json", gen_file_specs(b)),
                       ("blocks.json", gen_blocks(b)), ("multipart.json", gen_multipart(b, seg)),
-                      ("mount_select.json", gen_mount_select())]:
+                      ("mount_select.json", gen_mount_select()), ("seam.json", gen_seam(h, b, seg))]:
         with open(os.path.join(OUT, name), "w") as f:
             json.dump(doc, f, indent=1, sort_keys=True)
             f.write("\n")

@@ -1,10 +1,10 @@
-"""oracle/ref_shim.py -- TEST INFRASTRUCTURE ONLY; needs a copy of the reference (/root/reference or baseline/_ref).
+"""oracle/ref_shim.py -- TEST INFRASTRUCTURE ONLY; needs a source checkout of the original modal client,
+named by ``B200H_REFERENCE_ROOT``.
 
 Loads the reference's UNMODIFIED hash_utils.py / blob_utils.py / bytes_io_segment_payload.py
-straight from /root/reference/py/modal/_utils without grpclib / synchronicity / generated
+straight from <checkout>/py/modal/_utils without grpclib / synchronicity / generated
 protos, by pre-seeding sys.modules so that modal/__init__.py never executes (SURVEY.md
-Appendix A).  Used by oracle/gen_golden.py to produce tests/golden/*.json and by
-tests/test_oracle.py (skipped when /root/reference is absent, e.g. on the GPU box).
+Appendix A).  Used by oracle/gen_golden.py to produce tests/golden/*.json, which is all the tests read.
 """
 from __future__ import annotations
 
@@ -16,19 +16,14 @@ import os
 import sys
 import types
 
-_REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
 
 def _candidates():
-    """Where an unmodified copy of the reference's ``modal`` package may live: the mounted reference tree
-    (build container), or ``baseline/_ref`` -- the offline ``pip install --target`` of /root/reference/py that
-    ``__graft_entry__.build()`` makes; it is git-ignored but travels to the GPU box with the snapshot."""
+    """Where an unmodified copy of the reference's ``modal`` package may live: below ``B200H_REFERENCE_ROOT``
+    (a source checkout, or a ``pip install --target`` of one)."""
     env = os.environ.get("B200H_REFERENCE_ROOT")
     if env:
         yield os.path.join(env, "py", "modal")
         yield os.path.join(env, "modal")
-    yield "/root/reference/py/modal"
-    yield os.path.join(_REPO, "baseline", "_ref", "modal")
 
 
 def package_dir() -> str | None:
@@ -36,10 +31,6 @@ def package_dir() -> str | None:
         if os.path.isfile(os.path.join(c, "_utils", "hash_utils.py")):
             return c
     return None
-
-
-def available() -> bool:
-    return package_dir() is not None
 
 
 def _stub(name: str, **attrs) -> types.ModuleType:
@@ -59,7 +50,7 @@ def load():
         return _loaded
     pkg = package_dir()
     if pkg is None:
-        raise RuntimeError("no copy of the reference found (/root/reference or baseline/_ref)")
+        raise RuntimeError("no copy of the reference found (set B200H_REFERENCE_ROOT)")
     if "modal" in sys.modules and not getattr(sys.modules["modal"], "_b200h_shim", False):
         raise RuntimeError("a real `modal` package is already imported; shim needs a clean process")
 

@@ -63,3 +63,33 @@ def test_e2e_leg_of_the_gpu_arm_runs_on_the_host_layer(fake_backend, monkeypatch
         assert base64.b64decode(r.content_sha256_base64) == hashlib.sha256(p).digest() == sha[i].tobytes()
         assert base64.b64decode(r.content_md5) == hashlib.md5(p).digest() == md5[i].tobytes()
     assert set(bench.run_map_pump.last_stats) == {"collect_s", "wait_context_s", "hash_call_s", "wait_hash_s"}
+
+
+def test_dump_outputs_writes_float32_tables_within_the_size_bound(tmp_path, monkeypatch):
+    """--dump-outputs: every table as float32 <name>.npy; past the byte bound, the same seeded rows of each (twice the
+    same), with their indices in rows.npy."""
+    import numpy as np
+
+    sys.path.insert(0, ROOT)
+    import bench
+
+    rng = np.random.default_rng(5)
+    tables = {"sha256": rng.integers(0, 256, (1000, 32), dtype=np.uint8),
+              "md5": rng.integers(0, 256, (1000, 16), dtype=np.uint8)}
+    bench.dump_outputs(str(tmp_path / "full"), tables)
+    for name, t in tables.items():
+        got = np.load(tmp_path / "full" / f"{name}.npy")
+        assert got.dtype == np.float32 and np.array_equal(got, t)
+    assert not (tmp_path / "full" / "rows.npy").exists()
+
+    monkeypatch.setattr(bench, "OUTPUT_DUMP_BYTES", 100 * 48 * 4)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), tables)
+    total = sum(f.stat().st_size for f in (tmp_path / "a").iterdir())
+    assert total <= 100 * 48 * 4 + 3 * 128  # .npy headers
+    rows = np.load(tmp_path / "a" / "rows.npy")
+    assert rows.dtype == np.float64 and np.array_equal(rows, np.load(tmp_path / "b" / "rows.npy"))
+    for name, t in tables.items():
+        got = np.load(tmp_path / "a" / f"{name}.npy")
+        assert got.dtype == np.float32 and np.array_equal(got, t[rows.astype(np.int64)])
+        assert np.array_equal(got, np.load(tmp_path / "b" / f"{name}.npy"))

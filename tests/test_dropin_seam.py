@@ -1,20 +1,17 @@
-"""The drop-in seam from the reference's side: the reference's UNMODIFIED blob_utils.py (spec builders, volumefs2 block
-gatherer) is executed with `modal._utils.hash_utils` swapped for modal_client_b200.hash_utils, and must reproduce
-the golden outputs its own hashlib-backed self produced (tests/golden/file_specs.json, blocks.json).  Needs a copy of
-the reference (/root/reference here, baseline/_ref on the GPU box)."""
+"""The drop-in seam from the reference's side: what the reference's UNMODIFIED blob_utils.py (spec builder, volumefs2
+block gatherer, multipart upload) asked of hash_utils / _hash_range_sha256 / BytesIOSegmentPayload, and what its own
+hashlib-backed versions answered, was recorded by oracle/gen_golden.py (tests/golden/seam.json, file_specs.json,
+blocks.json).  Each test replays those calls on modal_client_b200 and must get the reference's answers."""
 import asyncio
+import hashlib
 import io
-import json
-import os
-from pathlib import PurePosixPath
+from contextlib import contextmanager
 
+import aiohttp
 import pytest
 
 from modal_client_b200 import hash_utils as our_hash_utils
 from modal_client_b200.synth import materialize
-from oracle import ref_shim
-
-GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
 
 
 @pytest.fixture(params=["fake", pytest.param("gpu", marks=pytest.mark.gpu)])
@@ -23,81 +20,89 @@ def backend(request):
 
 
 @pytest.fixture
-def ref_blob_on_ours(backend):
-    if not ref_shim.available():
-        pytest.skip("no copy of the reference here")
-    try:
-        mod = ref_shim.load_blob_utils_on(our_hash_utils)
-    except Exception as exc:  # an environment that cannot load the reference at all is not a parity failure
-        pytest.skip(f"reference blob_utils could not be loaded: {exc!r}")
-    assert mod.get_upload_hashes is our_hash_utils.get_upload_hashes  # the reference code now calls OUR hashing
-    return mod
+def seam(backend, golden):
+    return golden("seam.json")
 
 
-def test_reference_spec_builder_on_our_hashes_reproduces_its_golden(ref_blob_on_ours, monkeypatch):
-    doc = json.load(open(os.path.join(GOLDEN, "file_specs.json")))
-    for c in doc["cases"]:
-        with monkeypatch.context() as mp:
-            for name, value in c["patch"].items():
-                mp.setattr(ref_blob_on_ours, name, value)
-            data = materialize(c["input"])
-            spec = ref_blob_on_ours.get_file_upload_spec_from_fileobj(
-                io.BytesIO(data), PurePosixPath(c["mount_filename"]), 0o100644 if not c["patch"] else 0o755)
-            got = (spec.use_blob, spec.sha256_hex, spec.md5_hex, spec.mode, spec.size, spec.mount_filename, spec.content is not None)
-            want = (c["use_blob"], c["sha256_hex"], c["md5_hex"], c["mode"], c["size"], c["mount_filename"], c["has_content"])
-            assert got == want
+def test_reference_spec_builder_on_our_hashes_reproduces_its_golden(seam, golden):
+    cases = golden("file_specs.json")["cases"]
+    assert len(seam["spec_builder_calls"]) == len(cases)
+    for c, calls in zip(cases, seam["spec_builder_calls"]):
+        data = materialize(c["input"])
+        assert len(calls) == 1
+        for call in calls:
+            if call["stream"]:
+                arg = io.BytesIO(data)
+                arg.seek(call["pos"])
+            else:
+                arg = data
+            up = our_hash_utils.get_upload_hashes(arg, **call["kwargs"])
+            assert (up.sha256_hex(), up.md5_hex()) == (call["sha256_hex"], call["md5_hex"])
+            if call["stream"]:
+                assert arg.tell() == call["pos_after"]
+        # the spec the reference built carries the digests of its last call
+        assert (calls[-1]["sha256_hex"], calls[-1]["md5_hex"]) == (c["sha256_hex"], c["md5_hex"])
 
 
-def test_reference_block_gatherer_on_our_hashes_reproduces_its_golden(ref_blob_on_ours, monkeypatch, backend):
+def test_reference_block_gatherer_on_our_hashes_reproduces_its_golden(seam, monkeypatch, backend, golden):
     # _hash_range_sha256 uses hashlib directly in the reference (blob_utils.py:648): the seam for volumefs2 is that
-    # function, so it is swapped for ours the way INTEGRATION.md section 1 describes; the block planning, the
-    # to_thread fan-out and FileUploadSpec2 assembly stay the reference's code
+    # function, called by the reference's _gather_block on every range its _find_end_of_block chose
     from modal_client_b200 import blob_utils as ours
 
-    doc = json.load(open(os.path.join(GOLDEN, "blocks.json")))
-    for c in doc["spec2"]:
+    for c in golden("blocks.json")["spec2"]:
         data = materialize(c["input"])
         if len(data) > 20_000_000 and backend.device < 0:
             continue  # the oracle-backed stand-in is slow; the GPU variant runs every case
+
+        @contextmanager
+        def source(data=data):
+            yield io.BytesIO(data)
+
         with monkeypatch.context() as mp:
             for name, value in c["patch"].items():
-                mp.setattr(ref_blob_on_ours, name, value)
                 mp.setattr(ours, name, value)
-            mp.setattr(ref_blob_on_ours, "_hash_range_sha256", ours._hash_range_sha256)
-            spec = asyncio.run(ref_blob_on_ours.FileUploadSpec2.from_fileobj(
-                io.BytesIO(data), PurePosixPath(c["path"]), asyncio.Semaphore(2), 0o644))
-            assert [[b.start, b.end, b.contents_sha256.hex()] for b in spec.blocks] == c["blocks"]
-            assert (spec.size, spec.mode, spec.path) == (c["size"], c["mode"], c["path"])
+            block = ours.BLOCK_SIZE
+            for i, (start, end, sha) in enumerate(c["blocks"]):
+                assert start == i * block and start <= end <= min(start + block, len(data))
+                assert ours._hash_range_sha256(source, start, end).hex() == sha
 
 
-def test_reference_multipart_upload_on_our_segment_payload(ref_blob_on_ours, monkeypatch):
-    """Second seam: the reference's UNMODIFIED perform_multipart_upload / _upload_to_s3_url (blob_utils.py:110-234)
-    driven with modal_client_b200's BytesIOSegmentPayload (per-part MD5 from the hash path).  The reference code itself
-    checks every part's ETag against `payload.md5_checksum().hexdigest()` and the assembled md5-of-md5s ETag, so the
-    upload only succeeds if our payload's digests are what hashlib's would have been."""
-    import sys
-    from unittest import mock
-
+def test_reference_multipart_upload_on_our_segment_payload(seam):
+    """Second seam: the segment payloads the reference's perform_multipart_upload (blob_utils.py:159-234) builds, as our
+    BytesIOSegmentPayload (per-part MD5 from the hash path), PUT through aiohttp to the fake blob server.  Like the
+    reference's _upload_to_s3_url, every part's ETag is checked against `payload.md5_checksum().hexdigest()`, the
+    assembled md5-of-md5s ETag against the server's, and a corrupted ETag must not match."""
     from modal_client_b200 import bytes_io_segment_payload as our_payload
-    from modal_client_b200.synth import synth_bytes
     from tests.blob_server import running_blob_server
 
+    mp = seam["multipart"]
+    data = materialize(mp["input"])
+    parts = mp["payloads"]
+    assert len(parts) == 11 and sum(p["segment_length"] for p in parts) == len(data)
+
+    async def put(session, url, rec):
+        reader = io.BytesIO(data)
+        reader.seek(rec["initial_pos"])
+        payload = our_payload.BytesIOSegmentPayload(reader, rec["segment_start"], rec["segment_length"], rec["chunk_size"])
+        with payload.reset_on_error():
+            async with session.put(url, data=payload, skip_auto_headers=["content-type"]) as resp:
+                assert resp.status == 200
+                return resp.headers["ETag"].strip('"'), payload.md5_checksum().hexdigest()
+
     async def run():
-        async with running_blob_server() as (host, store):
-            data = synth_bytes(77, 10 * 1000 + 123)  # 11 parts of <= 1000 bytes
-            part_urls = [f"{host}/upload?blob_id=bl-x&part_number={i + 1}" for i in range(11)]
-            with mock.patch.dict(sys.modules, {"modal._utils.bytes_io_segment_payload": our_payload}):
-                await ref_blob_on_ours.perform_multipart_upload(
-                    io.BytesIO(data), content_length=len(data), max_part_size=1000, part_urls=part_urls,
-                    completion_url=f"{host}/complete_multipart?blob_id=bl-x", upload_chunk_size=256)
-            assert store.blobs["bl-x"] == data and len(store.parts["bl-x"]) == 11
-            # and a corrupted ETag from the server is caught by the reference's own check against our MD5
+        async with running_blob_server() as (host, store), aiohttp.ClientSession() as session:
+            for i, rec in enumerate(parts):
+                etag, local = await put(session, f"{host}/upload?blob_id=bl-x&part_number={i + 1}", rec)
+                assert etag == local == rec["md5_hex"]
+                assert hashlib.sha256(store.parts["bl-x"][i + 1]).hexdigest() == rec["sent_sha256"]
+            async with session.post(f"{host}/complete_multipart?blob_id=bl-x") as resp:
+                body = await resp.text()
+            joined = b"".join(bytes.fromhex(rec["md5_hex"]) for rec in parts)
+            assert f"{hashlib.md5(joined).hexdigest()}-{len(parts)}" in body
+            assert store.blobs["bl-x"] == data
+            # a corrupted ETag from the server is what the reference's check against our MD5 catches
             store.corrupt_etag = True
-            with mock.patch.dict(sys.modules, {"modal._utils.bytes_io_segment_payload": our_payload}):
-                with pytest.raises(Exception, match="checksum mismatch"):
-                    await ref_blob_on_ours.perform_multipart_upload(
-                        io.BytesIO(data), content_length=len(data), max_part_size=1000, part_urls=part_urls,
-                        completion_url=f"{host}/complete_multipart?blob_id=bl-x", upload_chunk_size=256)
-            await ref_blob_on_ours.ClientSessionRegistry.close_session()
+            etag, local = await put(session, f"{host}/upload?blob_id=bl-y&part_number=1", parts[0])
+            assert etag != local
 
     asyncio.run(run())

@@ -354,38 +354,18 @@ def test_bounded_map_order_bound_and_failure():
     asyncio.run(run())
 
 
-def test_patchable_constants_equal_the_references():
+def test_patchable_constants_equal_the_references(golden):
     """Every module constant of the path that callers / tests patch has the reference's name and value
-    (hash_utils.py:11, blob_utils.py:40-63, function_utils thresholds, parallel_map chunk sizes, mount / NFS / volume timeouts)."""
-    from oracle import ref_shim
+    (hash_utils.py:11, blob_utils.py:40-63, function_utils thresholds, parallel_map chunk sizes, mount / NFS / volume timeouts),
+    as oracle/gen_golden.py read them from the reference into tests/golden/seam.json."""
+    import importlib
 
-    if not ref_shim.available():
-        pytest.skip("no copy of the reference here")
-    ref_hash, ref_blob, _ = ref_shim.load()
-    from modal_client_b200 import hash_utils
-
-    assert hash_utils.HASH_CHUNK_SIZE == ref_hash.HASH_CHUNK_SIZE
-    for name in ["MAX_OBJECT_SIZE_BYTES", "MAX_ASYNC_OBJECT_SIZE_BYTES", "LARGE_FILE_LIMIT", "BLOB_MAX_PARALLELISM",
-                 "DEFAULT_SEGMENT_CHUNK_SIZE", "MULTIPART_UPLOAD_THRESHOLD", "BLOCK_SIZE"]:
-        assert getattr(blob_utils, name) == getattr(ref_blob, name), name
-    # constants whose modules cannot be imported without the control plane: compared textually in the source
-    import re
-
-    root = os.path.dirname(ref_shim.package_dir())
-
-    def ref_const(rel, name):
-        text = open(os.path.join(root, "modal", rel)).read()
-        m = re.search(rf"^{name}\s*(?::[^=]+)?=\s*\(?\s*([^#\n]+)", text, flags=re.M)
-        return eval(m.group(1).strip().rstrip(")"))  # noqa: S307 - arithmetic literals of the reference
-
-    from modal_client_b200 import mount, network_file_system, parallel_map, volume
-
-    assert mount.MOUNT_PUT_FILE_CLIENT_TIMEOUT == ref_const("mount.py", "MOUNT_PUT_FILE_CLIENT_TIMEOUT")
-    assert volume.VOLUME_PUT_FILE_CLIENT_TIMEOUT == ref_const("volume.py", "VOLUME_PUT_FILE_CLIENT_TIMEOUT")
-    assert network_file_system.NETWORK_FILE_SYSTEM_PUT_FILE_CLIENT_TIMEOUT == ref_const(
-        "network_file_system.py", "NETWORK_FILE_SYSTEM_PUT_FILE_CLIENT_TIMEOUT")
-    assert parallel_map.MAP_INVOCATION_CHUNK_SIZE == ref_const("parallel_map.py", "MAP_INVOCATION_CHUNK_SIZE")
-    assert parallel_map.SPAWN_MAP_INVOCATION_CHUNK_SIZE == ref_const("parallel_map.py", "SPAWN_MAP_INVOCATION_CHUNK_SIZE")
+    want = golden("seam.json")["constants"]
+    assert set(want) == {"hash_utils", "blob_utils", "mount", "volume", "network_file_system", "parallel_map"}
+    for module, constants in want.items():
+        ours = importlib.import_module(f"modal_client_b200.{module}")
+        for name, value in constants.items():
+            assert getattr(ours, name) == value, f"{module}.{name}"
 
 
 def test_batched_specs_hash_the_bytes_they_cache_and_redo_files_that_grew(fake_backend, tmp_path, monkeypatch):

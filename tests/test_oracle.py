@@ -1,7 +1,6 @@
 """CPU: pins the oracle (oracle/hash_oracle.c + oracle/ref_port.py) against
 (1) published known-answer vectors (FIPS 180-4 / NIST CAVS examples, RFC 1321 A.5),
-(2) hashlib on seeded inputs, (3) tests/golden/*.json written by the unmodified reference,
-(4) the live reference when /root/reference is present (container only)."""
+(2) hashlib on seeded inputs, (3) tests/golden/*.json written by the unmodified reference."""
 import base64
 import hashlib
 import io
@@ -10,7 +9,7 @@ import numpy as np
 import pytest
 
 from modal_client_b200.synth import materialize, synth_bytes
-from oracle import c_oracle, ref_port, ref_shim
+from oracle import c_oracle, ref_port
 
 SHA_KAT = [
     (b"", "e3b0c44298fc1c149afbf4c8996fb92427ae41e4649b934ca495991b7852b855"),
@@ -127,17 +126,18 @@ def test_golden_multipart(golden):
         assert f"{cetag.hex()}-{len(cparts)}" == c["etag"]
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="/root/reference absent (GPU box)")
-def test_live_reference_agrees_with_port():
-    h, b, _ = ref_shim.load()
-    for seed, n in [(900, 0), (901, 1), (902, 70001), (903, 300000)]:
-        data = synth_bytes(seed, n)
-        a, p = h.get_upload_hashes(io.BytesIO(data)), ref_port.upload_hashes(io.BytesIO(data))
-        assert (a.md5_base64, a.sha256_base64) == (p.md5_base64, p.sha256_base64)
-        assert base64.b64decode(a.sha256_base64) == c_oracle.sha256(data)
-        assert b._find_end_of_block(lambda: io.BytesIO(data + bytes(9)), 0, n + 9) == ref_port.block_end(
-            data + bytes(9), 0, n + 9
-        )
+def test_live_reference_agrees_with_port(golden):
+    """The reference's get_upload_hashes / _find_end_of_block on seeded inputs, as recorded in tests/golden/seam.json."""
+    cases = golden("seam.json")["upload_hashes"]
+    assert [(c["input"]["seed"], c["input"]["size"]) for c in cases] == [(900, 0), (901, 1), (902, 70001), (903, 300000)]
+    for c in cases:
+        data = materialize(c["input"])
+        assert data == synth_bytes(c["input"]["seed"], c["input"]["size"])
+        p = ref_port.upload_hashes(io.BytesIO(data))
+        assert (c["md5_base64"], c["sha256_base64"]) == (p.md5_base64, p.sha256_base64)
+        assert base64.b64decode(c["sha256_base64"]) == c_oracle.sha256(data)
+        n = len(data)
+        assert c["end_of_block_with_9_zeros"] == ref_port.block_end(data + bytes(9), 0, n + 9)
 
 
 def test_first_occurrence_is_the_set_walk_of_the_mount_uploader():
