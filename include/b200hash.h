@@ -198,6 +198,51 @@ uint64_t b200h_plan_sync_count(b200h_ctx* ctx);
 int b200h_profile_enable(b200h_ctx* ctx, int on);
 int b200h_profile_read(b200h_ctx* ctx, double* hash_kernel_ms, uint64_t* hash_kernel_launches);
 
+/* ---- device groups: one process, several GPUs ------------------------------------------------------ */
+
+/* A group is one context per listed device (a device may repeat: {0, 0} is two contexts on one GPU), driven as one.
+ * b200h_group_hash_batch_host / _hash_files deal a batch over the members by bytes (b200h_group_split_preview), every
+ * member hashes its share on its own thread at the same time, and the rows land at the caller's message indices.
+ * Members on one NUMA node divide its CPUs between their packer and reader teams.  Group calls are thread-safe.
+ * Everything else (stat_files, dedupe_*, hash_fixed_parts, streams, host_alloc, the *_device entry points) is not
+ * split: call it on b200h_group_member(g, 0), the "home" member.  Its host_alloc memory is portable, so every member
+ * DMAs it directly. */
+typedef struct b200h_group b200h_group;
+
+/* min_share_bytes: a batch is split over k = min(members, messages, max(1, total bytes / min_share_bytes)) members
+ * (0 = the default, B200H_GROUP_MIN_SHARE).  pinned_bytes / device_bytes size every member as in b200h_create. */
+#define B200H_GROUP_MIN_SHARE (256ull << 20)
+int b200h_group_create(const int* devices, int ndevices, size_t pinned_bytes, size_t device_bytes,
+                       uint64_t min_share_bytes, b200h_group** out);
+void b200h_group_destroy(b200h_group* g);
+/* g may be NULL: the message of the last failed b200h_group_create on this thread.  A failed batch names the first
+ * failing member ("member 1 (cuda:0): ..."); the other members finish their shares, the outputs are unspecified and
+ * the group stays usable. */
+const char* b200h_group_last_error(b200h_group* g);
+int b200h_group_size(b200h_group* g);
+b200h_ctx* b200h_group_member(b200h_group* g, int i); /* owned by the group; member 0 = "home" */
+/* As b200h_hash_batch_host.  With k == 1 this IS that call on the home member (combining queue included).  Outputs
+ * may be host or device memory; device outputs must all be on one device (the table device), B200H_E_INVALID
+ * otherwise: each member hashes into its own HBM and scatter_rows_kernel writes its rows into the table, over peer
+ * access where the devices allow it (enabled for this process's contexts only), else after a cudaMemcpyPeerAsync. */
+int b200h_group_hash_batch_host(b200h_group* g, const uint8_t* base, const uint64_t* offsets, const uint64_t* lengths,
+                                uint64_t n, uint32_t flags, uint8_t* sha256_out, uint8_t* md5_out,
+                                uint64_t* trimmed_len_out);
+/* As b200h_hash_files; with part_len > 0 the parts are dealt, so one file's blocks may land on several members. */
+int b200h_group_hash_files(b200h_group* g, const char* const* paths, uint64_t n, const uint64_t* sizes,
+                           uint64_t part_len, uint32_t flags, uint8_t* sha256_out, uint8_t* md5_out,
+                           uint64_t* trimmed_len_out);
+/* What the last batch call did, per member (arrays of b200h_group_size entries, each may be NULL): messages, payload
+ * bytes, bytes that went through the member's pinned staging ring (0 = DMAed straight from the caller's page-locked
+ * memory) and wall milliseconds spent inside the member.  Members the batch did not use report zeros. */
+int b200h_group_last_split(b200h_group* g, uint64_t* messages_out, uint64_t* bytes_out, uint64_t* staged_bytes_out,
+                           double* busy_ms_out);
+/* The split decision alone: owner_out[n] = member of every message, *members_used_out = k.  Messages are sorted by
+ * length (longest first, stable) and dealt over members 0..k-1 in boustrophedon order (0..k-1, k-1..0, ...).  Pure
+ * host arithmetic: no group, no GPU.  min_share_bytes 0 = B200H_GROUP_MIN_SHARE. */
+int b200h_group_split_preview(const uint64_t* lengths, uint64_t n, int nmembers, uint64_t min_share_bytes,
+                              uint32_t* owner_out, int* members_used_out);
+
 #ifdef __cplusplus
 }
 #endif

@@ -33,6 +33,8 @@ ABI_SYMBOLS = (
     "b200h_profile_enable", "b200h_profile_read", "b200h_dedupe_host", "b200h_dedupe_device",
     "b200h_last_outlier_count", "b200h_hash_batch_device_hl", "b200h_combine_stats", "b200h_plan_sync_count",
     "b200h_stream_copy", "b200h_stream_copy_isa", "b200h_plan_preview", "b200h_pack_preview",
+    "b200h_group_create", "b200h_group_destroy", "b200h_group_last_error", "b200h_group_size", "b200h_group_member",
+    "b200h_group_hash_batch_host", "b200h_group_hash_files", "b200h_group_last_split", "b200h_group_split_preview",
 )
 
 
@@ -42,7 +44,8 @@ class B200HashError(RuntimeError):
 
 def build_library(force: bool = False, verbose: bool = False) -> str:
     srcs = [os.path.join(CSRC, f) for f in ("b200hash_kernels.cu", "b200hash_dedupe.cu", "b200hash_api.cu",
-                                            "b200blob_host.cpp", "b200pack_copy.cpp", "b200hash_kernels.cuh", "b200pack_team.h")]
+                                            "b200hash_group.cu", "b200hash_internal.h", "b200blob_host.cpp",
+                                            "b200pack_copy.cpp", "b200hash_kernels.cuh", "b200pack_team.h")]
     srcs += [os.path.join(os.path.dirname(_PKG), "include", h) for h in ("b200hash.h", "b200blob.h")]
     stale = not os.path.exists(LIB_PATH) or any(os.path.getmtime(s) > os.path.getmtime(LIB_PATH) for s in srcs)
     if force or stale:
@@ -134,6 +137,24 @@ def load_library() -> ctypes.CDLL:
         L.b200h_plan_preview.restype = i32
         L.b200h_pack_preview.argtypes = [vp, vp, vp, u64, vp, u64, u64, i32, vp]
         L.b200h_pack_preview.restype = i32
+        L.b200h_group_create.argtypes = [vp, i32, sz, sz, u64, ctypes.POINTER(vp)]
+        L.b200h_group_create.restype = i32
+        L.b200h_group_destroy.argtypes = [vp]
+        L.b200h_group_destroy.restype = None
+        L.b200h_group_last_error.argtypes = [vp]
+        L.b200h_group_last_error.restype = ctypes.c_char_p
+        L.b200h_group_size.argtypes = [vp]
+        L.b200h_group_size.restype = i32
+        L.b200h_group_member.argtypes = [vp, i32]
+        L.b200h_group_member.restype = vp
+        L.b200h_group_hash_batch_host.argtypes = [vp, vp, vp, vp, u64, u32, vp, vp, vp]
+        L.b200h_group_hash_batch_host.restype = i32
+        L.b200h_group_hash_files.argtypes = [vp, vp, u64, vp, u64, u32, vp, vp, vp]
+        L.b200h_group_hash_files.restype = i32
+        L.b200h_group_last_split.argtypes = [vp, vp, vp, vp, vp]
+        L.b200h_group_last_split.restype = i32
+        L.b200h_group_split_preview.argtypes = [vp, u64, i32, u64, vp, ctypes.POINTER(i32)]
+        L.b200h_group_split_preview.restype = i32
         _lib = L
         return L
 
@@ -159,6 +180,19 @@ def plan_preview(lengths, flags: int = SHA256 | MD5, sm_count: int = 148) -> tup
     if rc != 0:
         raise B200HashError(f"b200h_plan_preview failed ({rc})")
     return c.value, l.value
+
+
+def group_split_preview(lengths, nmembers: int, min_share_bytes: int = 0) -> tuple[np.ndarray, int]:
+    """(owner uint32[n], members used k): how a device group of ``nmembers`` deals a batch with these lengths --
+    the library's own split (no group, no GPU).  ``min_share_bytes`` 0 = the library default."""
+    L = load_library()
+    ln = np.ascontiguousarray(lengths, dtype=np.uint64)
+    owner = np.empty(max(ln.size, 1), np.uint32)
+    k = ctypes.c_int()
+    rc = L.b200h_group_split_preview(_np_ptr(ln), ln.size, nmembers, min_share_bytes, _np_ptr(owner), ctypes.byref(k))
+    if rc != 0:
+        raise B200HashError(f"b200h_group_split_preview failed ({rc})")
+    return owner[: ln.size], k.value
 
 
 def pack_preview(base, offsets, lengths, threads: int = 16, slot_bytes: int = 256 << 20, dst: np.ndarray | None = None):
@@ -284,13 +318,15 @@ class Context:
         sha = np.empty((n, 32 * wide), np.uint8) if (flags & SHA256 and not out_sha) else None
         md5 = np.empty((n, 16 * wide), np.uint8) if (flags & MD5 and not out_md5) else None
         trimmed = None if out_trimmed else np.empty(n, np.uint64)
-        rc = self._L.b200h_hash_batch_host(self._h, bp, _np_ptr(off), _np_ptr(ln), n, flags,
-                                           ctypes.c_void_p(out_sha) if out_sha else _np_ptr(sha),
-                                           ctypes.c_void_p(out_md5) if out_md5 else _np_ptr(md5),
-                                           ctypes.c_void_p(out_trimmed) if out_trimmed else _np_ptr(trimmed))
-        self._check(rc, "b200h_hash_batch_host")
+        self._batch_host(bp, _np_ptr(off), _np_ptr(ln), n, flags,
+                         ctypes.c_void_p(out_sha) if out_sha else _np_ptr(sha),
+                         ctypes.c_void_p(out_md5) if out_md5 else _np_ptr(md5),
+                         ctypes.c_void_p(out_trimmed) if out_trimmed else _np_ptr(trimmed))
         del keep
         return sha, md5, trimmed
+
+    def _batch_host(self, *args):
+        self._check(self._L.b200h_hash_batch_host(self._h, *args), "b200h_hash_batch_host")
 
     def hash_buffers(self, bufs: Sequence, flags: int = SHA256 | MD5):
         """Hash many separate bytes-like objects without packing them in Python: their addresses go to
@@ -370,10 +406,11 @@ class Context:
         sha = np.empty((rows, 32 * wide), np.uint8) if flags & SHA256 else None
         md5 = np.empty((rows, 16 * wide), np.uint8) if flags & MD5 else None
         trimmed = np.empty(rows, np.uint64)
-        rc = self._L.b200h_hash_files(self._h, arr, n, _np_ptr(sizes), part_len, flags, _np_ptr(sha), _np_ptr(md5),
-                                      _np_ptr(trimmed))
-        self._check(rc, "b200h_hash_files")
+        self._files(arr, n, _np_ptr(sizes), part_len, flags, _np_ptr(sha), _np_ptr(md5), _np_ptr(trimmed))
         return sha, md5, trimmed
+
+    def _files(self, *args):
+        self._check(self._L.b200h_hash_files(self._h, *args), "b200h_hash_files")
 
     # -- dedupe of a digest table (first occurrence of every content)
     def dedupe(self, keys: np.ndarray) -> tuple[np.ndarray, int]:
@@ -401,6 +438,62 @@ class Context:
 
     def stream(self, flags: int = SHA256 | MD5) -> "DigestStream":
         return DigestStream(self, flags)
+
+
+class DeviceGroup(Context):
+    """One context per listed device, driven as one (include/b200hash.h, device groups).  ``hash_batch_host`` (and so
+    ``hash_buffers``) and ``hash_files`` deal each batch over the members by bytes and hash the shares at the same time;
+    every other method runs on the home member (``devices[0]``), whose handle this object carries as a Context.
+    ``devices=None`` means every visible device; a device may repeat.  ``min_share_bytes`` 0 = the library default."""
+
+    def __init__(self, devices: Sequence[int] | None = None, pinned_bytes: int = 0, device_bytes: int = 0,
+                 min_share_bytes: int = 0):
+        self._L = load_library()
+        if devices is None:
+            devices = list(range(self._L.b200h_device_count()))
+        devs = (ctypes.c_int * max(len(devices), 1))(*devices)
+        g = ctypes.c_void_p()
+        rc = self._L.b200h_group_create(devs, len(devices), pinned_bytes, device_bytes, min_share_bytes, ctypes.byref(g))
+        if rc != 0:
+            msg = (self._L.b200h_group_last_error(None) or b"").decode()
+            raise B200HashError(f"b200h_group_create(devices={list(devices)}) failed ({rc}): {msg}")
+        self._g = g
+        self.devices = [int(d) for d in devices]
+        self._members = [ctypes.c_void_p(self._L.b200h_group_member(g, i)) for i in range(len(self.devices))]
+        self._h = self._members[0]  # borrowed: the group owns it
+        self.device = self.devices[0]
+
+    def _gcheck(self, rc: int, what: str):
+        if rc != 0:
+            msg = (self._L.b200h_group_last_error(self._g) or b"").decode()
+            raise B200HashError(f"{what} failed ({rc}): {msg}")
+
+    def _batch_host(self, *args):
+        self._gcheck(self._L.b200h_group_hash_batch_host(self._g, *args), "b200h_group_hash_batch_host")
+
+    def _files(self, *args):
+        self._gcheck(self._L.b200h_group_hash_files(self._g, *args), "b200h_group_hash_files")
+
+    def close(self):
+        if getattr(self, "_g", None):
+            self._L.b200h_group_destroy(self._g)
+        self._g = None
+        self._h = None  # never destroyed on its own: it belonged to the group
+
+    @property
+    def launch_count(self) -> int:
+        return sum(int(self._L.b200h_launch_count(h)) for h in self._members) if getattr(self, "_g", None) else 0
+
+    def last_split(self) -> list[dict]:
+        """Per member, what the last batch call did: device, messages, payload bytes, bytes that went through the
+        member's pinned staging ring (0 = DMAed straight from page-locked memory), wall ms inside the member."""
+        m = len(self.devices)
+        msgs, nbytes, staged = np.zeros(m, np.uint64), np.zeros(m, np.uint64), np.zeros(m, np.uint64)
+        ms = np.zeros(m, np.float64)
+        self._gcheck(self._L.b200h_group_last_split(self._g, _np_ptr(msgs), _np_ptr(nbytes), _np_ptr(staged), _np_ptr(ms)),
+                     "b200h_group_last_split")
+        return [{"device": d, "messages": int(a), "bytes": int(b), "staged_bytes": int(s), "busy_ms": float(t)}
+                for d, a, b, s, t in zip(self.devices, msgs, nbytes, staged, ms)]
 
 
 class DigestStream:

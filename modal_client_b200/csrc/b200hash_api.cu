@@ -33,6 +33,7 @@
 #include <vector>
 
 #include "../../include/b200hash.h"
+#include "b200hash_internal.h"
 #include "b200hash_kernels.cuh"
 #include "b200pack_team.h"
 
@@ -152,6 +153,7 @@ struct b200h_ctx {
     uint64_t* h_meta = nullptr;  // pinned: offsets then lengths
     size_t h_meta_cap = 0;       // in uint64 elements
     uint64_t launches = 0;
+    std::atomic<uint64_t> staged_bytes{0};  // bytes packed / read into the pinned staging ring (the rest: DMA from source)
     bool profiling = false;
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> prof_events;
     double prof_ms = 0.0;
@@ -542,9 +544,14 @@ void pack_parallel(PackTeam& team, int threads, const Source& src, const uint64_
     team.run(t, cpus, work);
 }
 
+// A sparse selection of page-locked memory whose messages average at least this many bytes is DMAed one message at a
+// time (gather_pinned): one cudaMemcpyAsync costs a few microseconds, a 1 MiB message ~20 us of PCIe.
+constexpr uint64_t kGatherMinAvg = uint64_t(1) << 20;
+
 int hash_batch_host_impl(b200h_ctx* ctx, const uint8_t* base, const uint64_t* off, const uint64_t* len, uint64_t n,
                          uint32_t flags, uint8_t* sha_out, uint8_t* md5_out, uint64_t* trim_out, uint8_t* etag_out,
-                         const char* const* paths = nullptr, const uint64_t* file_of = nullptr) {
+                         const char* const* paths = nullptr, const uint64_t* file_of = nullptr,
+                         bool gather_pinned = false) {
     if (n == 0) return 0;
     std::atomic<int> io_errno{0};
     std::atomic<uint64_t> io_file{0};
@@ -564,7 +571,9 @@ int hash_batch_host_impl(b200h_ctx* ctx, const uint8_t* base, const uint64_t* of
     // (Only when the messages cover most of the span they sit in: a wave DMAs its whole [min offset, max end) span,
     // so a sparse selection -- one rank's interleaved shard of a shared buffer -- would copy the gaps too; those
     // are gathered through the staging ring like pageable memory.)
-    bool direct = false;
+    // (gather_pinned: a device group member's share, dealt from the whole batch, is sparse by construction; large
+    // messages are then DMAed one by one into the packed wave layout instead.)
+    bool direct = false, gather = false;
     if (base && !paths) {
         cudaPointerAttributes at;
         if (cudaPointerGetAttributes(&at, base) == cudaSuccess) direct = (at.type == cudaMemoryTypeHost);
@@ -576,7 +585,8 @@ int hash_batch_host_impl(b200h_ctx* ctx, const uint8_t* base, const uint64_t* of
                 hi = std::max(hi, off[i] + len[i]);
                 payload += len[i];
             }
-            if (hi - lo > payload + payload / 4 + (uint64_t(16) << 20)) direct = false;
+            if (hi - lo > payload + payload / 4 + (uint64_t(16) << 20))
+                direct = gather = gather_pinned && payload >= n * kGatherMinAvg;
         }
     }
 
@@ -608,7 +618,7 @@ int hash_batch_host_impl(b200h_ctx* ctx, const uint8_t* base, const uint64_t* of
                 i += 1;
                 continue;
             }
-            if (direct) {
+            if (direct && !gather) {
                 uint64_t lo = off[i], hi = off[i] + len[i];
                 uint64_t j = i + 1;
                 for (; j < n; ++j) {
@@ -675,7 +685,12 @@ int hash_batch_host_impl(b200h_ctx* ctx, const uint8_t* base, const uint64_t* of
         Source seg_src = src;
         seg_src.off = &seg_off1;
         seg_src.file_of = file_of ? &seg_file1 : nullptr;
-        if (direct) {
+        if (gather && !w.seg) {
+            for (uint64_t k = w.i0; k < w.i1; ++k)
+                if (len[k])
+                    CU_TRY(ctx, cudaMemcpyAsync(ctx->dwave[slot] + doff[k], base + off[k], len[k], cudaMemcpyHostToDevice,
+                                                ctx->s_copy));
+        } else if (direct) {
             const uint8_t* from = w.seg ? base + off[w.i0] + w.seg_start : base + w.src_lo;
             if (w.bytes) CU_TRY(ctx, cudaMemcpyAsync(ctx->dwave[slot], from, w.bytes, cudaMemcpyHostToDevice, ctx->s_copy));
         } else {
@@ -698,6 +713,7 @@ int hash_batch_host_impl(b200h_ctx* ctx, const uint8_t* base, const uint64_t* of
                 }
                 CU_TRY(ctx, cudaMemcpyAsync(ctx->dwave[slot] + lo, ctx->pin[pin_slot], hi - lo, cudaMemcpyHostToDevice,
                                             ctx->s_copy));
+                ctx->staged_bytes += hi - lo;
                 CU_TRY(ctx, cudaEventRecord(ctx->ev_pin[pin_slot], ctx->s_copy));
                 pin_used[pin_slot] = true;
                 pin_slot ^= 1;
@@ -867,6 +883,13 @@ int b200h_device_count(void) {
 const char* b200h_last_error(b200h_ctx* ctx) { return ctx ? ctx->err.c_str() : g_create_error.c_str(); }
 
 int b200h_create(int device, size_t pinned_bytes, size_t device_bytes, b200h_ctx** out) {
+    return b200h::create_member(device, pinned_bytes, device_bytes, nullptr, 0, out);
+}
+
+}  // extern "C"
+
+int b200h::create_member(int device, size_t pinned_bytes, size_t device_bytes, const int* group_devices, int ngroup,
+                         b200h_ctx** out) {
     if (!out) return fail(nullptr, B200H_E_INVALID, "out is NULL");
     *out = nullptr;
     int ndev = 0;
@@ -957,6 +980,18 @@ int b200h_create(int device, size_t pinned_bytes, size_t device_bytes, b200h_ctx
             share = std::max(4u, share / std::max(1u, per_node));
         }
     }
+    // The members of a device group that sit on this device's NUMA node (this one included) divide its CPUs the same
+    // way; without a known node every member shares the whole host.
+    if (ngroup > 1) {
+        unsigned sharers = 0;
+        for (int g = 0; g < ngroup; ++g) {
+            cpu_set_t other;
+            if (!ctx->node_cpus_valid || group_devices[g] == device ||
+                (gpu_node_cpus(group_devices[g], &other) && CPU_EQUAL(&other, &ctx->node_cpus)))
+                ++sharers;
+        }
+        share = std::max(4u, share / std::max(1u, sharers));
+    }
     ctx->pack_threads = (int)std::min(16u, std::max(2u, share / 2));  // 16: measured best on 2x Xeon 8562Y+ (8..64 tried)
     if (const char* e = getenv("B200H_PACK_THREADS")) ctx->pack_threads = std::max(1, atoi(e));
     ctx->io_threads = (int)std::min(16u, std::max(1u, share));  // measured: 16 > 32 > 64 > 128 (kernel-side contention)
@@ -971,6 +1006,38 @@ int b200h_create(int device, size_t pinned_bytes, size_t device_bytes, b200h_ctx
     *out = ctx;
     return 0;
 }
+
+void b200h::file_messages(const uint64_t* sizes, uint64_t n, uint64_t part_len, std::vector<uint64_t>& off,
+                          std::vector<uint64_t>& len, std::vector<uint64_t>& file_of) {
+    for (uint64_t f = 0; f < n; ++f) {
+        if (part_len == 0) {
+            off.push_back(0);
+            len.push_back(sizes[f]);
+            file_of.push_back(f);
+        } else {
+            for (uint64_t o = 0; o < sizes[f]; o += part_len) {
+                off.push_back(o);
+                len.push_back(std::min(part_len, sizes[f] - o));
+                file_of.push_back(f);
+            }
+        }
+    }
+}
+
+uint64_t b200h::staged_bytes(b200h_ctx* ctx) { return ctx->staged_bytes.load(); }
+
+int b200h::hash_share(b200h_ctx* ctx, const uint8_t* base, const uint64_t* off, const uint64_t* len, uint64_t n,
+                      uint32_t flags, uint8_t* sha_out, uint8_t* md5_out, uint64_t* trim_out, const char* const* paths,
+                      const uint64_t* file_of, uint64_t* staged_out) {
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    const uint64_t staged0 = ctx->staged_bytes;
+    const int rc = hash_batch_host_impl(ctx, base, off, len, n, flags & kPublicFlags, sha_out, md5_out, trim_out, nullptr,
+                                        paths, file_of, /*gather_pinned=*/true);
+    *staged_out = ctx->staged_bytes - staged0;
+    return rc;
+}
+
+extern "C" {
 
 void b200h_destroy(b200h_ctx* ctx) {
     if (!ctx) return;
@@ -1142,21 +1209,8 @@ int b200h_hash_files(b200h_ctx* ctx, const char* const* paths, uint64_t n, const
     B200H_RANGE("b200h_hash_files");
     std::lock_guard<std::mutex> lk(ctx->mu);
     if (n && (!paths || !sizes)) return fail(ctx, B200H_E_INVALID, "paths/sizes must not be NULL");
-    // message list: one per file (part_len == 0) or one per part_len-sized part, file-major
     std::vector<uint64_t> off, len, file_of;
-    for (uint64_t f = 0; f < n; ++f) {
-        if (part_len == 0) {
-            off.push_back(0);
-            len.push_back(sizes[f]);
-            file_of.push_back(f);
-        } else {
-            for (uint64_t o = 0; o < sizes[f]; o += part_len) {
-                off.push_back(o);
-                len.push_back(std::min(part_len, sizes[f] - o));
-                file_of.push_back(f);
-            }
-        }
-    }
+    b200h::file_messages(sizes, n, part_len, off, len, file_of);
     if (off.empty()) return 0;
     return hash_batch_host_impl(ctx, nullptr, off.data(), len.data(), off.size(), flags & kPublicFlags, sha256_out,
                                 md5_out, trimmed_len_out, nullptr, paths, file_of.data());

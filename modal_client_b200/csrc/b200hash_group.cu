@@ -1,0 +1,533 @@
+// b200hash_group.cu -- device groups: one process hashes its batches on several GPUs (C ABI: include/b200hash.h).
+//
+// A group owns one context per listed device and one parked worker thread per member.  A batch is dealt over the
+// members by bytes (split_owner), every worker hashes its member's share through that member's context, and the rows
+// are scattered back to the caller's message indices: with memcpy for host outputs, with scatter_rows_kernel for
+// device outputs.  A worker only ever touches its own member, so no thread holds two member mutexes at once and
+// concurrent group calls cannot deadlock; the calling thread holds none while it waits.
+#include <cuda_runtime.h>
+#include <stdint.h>
+
+#include <algorithm>
+#include <chrono>
+#include <condition_variable>
+#include <cstring>
+#include <deque>
+#include <functional>
+#include <memory>
+#include <mutex>
+#include <numeric>
+#include <string>
+#include <thread>
+#include <vector>
+
+#include "../../include/b200hash.h"
+#include "b200hash_internal.h"
+
+namespace {
+
+thread_local std::string g_group_create_error;
+
+// dst[idx[r] * width + b] = src[r * width + b] for the `rows` rows of one member's share: raw or hex digest rows and
+// 8-byte hashed lengths into the caller's table.  dst may be another device's memory reached over peer access.
+__global__ void scatter_rows_kernel(const uint8_t* __restrict__ src, const uint64_t* __restrict__ idx, uint64_t rows,
+                                    uint32_t width, uint8_t* __restrict__ dst) {
+    const uint64_t total = rows * width;
+    for (uint64_t t = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; t < total; t += (uint64_t)gridDim.x * blockDim.x) {
+        const uint64_t r = t / width;
+        dst[idx[r] * width + (t - r * width)] = src[t];
+    }
+}
+
+// A member's thread: started with the group, parked on a condition variable between jobs, joined in destroy.
+class Worker {
+public:
+    Worker() : th_([this] { loop(); }) {}
+    Worker(const Worker&) = delete;
+    Worker& operator=(const Worker&) = delete;
+    ~Worker() {
+        {
+            std::lock_guard<std::mutex> lk(m_);
+            stop_ = true;
+        }
+        cv_.notify_one();
+        th_.join();
+    }
+    void post(std::function<void()> job) {
+        {
+            std::lock_guard<std::mutex> lk(m_);
+            q_.push_back(std::move(job));
+        }
+        cv_.notify_one();
+    }
+
+private:
+    void loop() {
+        for (;;) {
+            std::function<void()> job;
+            {
+                std::unique_lock<std::mutex> lk(m_);
+                cv_.wait(lk, [&] { return stop_ || !q_.empty(); });
+                if (q_.empty()) return;
+                job = std::move(q_.front());
+                q_.pop_front();
+            }
+            job();
+        }
+    }
+
+    std::mutex m_;
+    std::condition_variable cv_;
+    std::deque<std::function<void()>> q_;
+    bool stop_ = false;
+    std::thread th_;  // last: the thread starts once the members above exist
+};
+
+struct DevScratch {
+    int device = -1;
+    uint8_t* p = nullptr;
+    size_t cap = 0;
+};
+
+// Everything below `worker` is touched by the worker thread only.
+struct Member {
+    b200h_ctx* ctx = nullptr;
+    int device = 0;
+    std::unique_ptr<Worker> worker;
+    cudaStream_t st = nullptr;          // on `device`
+    DevScratch share;                   // on `device`: the share's device output columns, then its row indices
+    DevScratch staged;                  // on the table device when it cannot reach `share` over peer access
+    cudaStream_t st_table = nullptr;    // on staged.device
+    std::vector<signed char> peer;      // per table device: -1 not asked yet, 0 no peer access, 1 enabled
+};
+
+// The output columns of a batch: sha256 | md5 | hashed length.
+struct Columns {
+    uint8_t* out[3] = {nullptr, nullptr, nullptr};
+    uint32_t width[3] = {0, 0, 8};
+    bool on_device[3] = {false, false, false};
+    int table_device = -1;
+};
+
+struct Share {
+    std::vector<uint64_t> idx, off, len, file_of;
+    uint64_t bytes = 0, staged = 0;
+    double ms = 0.0;
+    int rc = 0;
+    std::string err;
+};
+
+}  // namespace
+
+struct b200h_group {
+    std::vector<std::unique_ptr<Member>> members;
+    uint64_t min_share = B200H_GROUP_MIN_SHARE;
+    std::mutex mu;  // err and the last split
+    std::string err;
+    std::vector<uint64_t> last_messages, last_bytes, last_staged;
+    std::vector<double> last_ms;
+};
+
+namespace {
+
+using Clock = std::chrono::steady_clock;
+
+double ms_since(Clock::time_point t0) { return std::chrono::duration<double, std::milli>(Clock::now() - t0).count(); }
+
+std::string cuda_msg(const char* what, cudaError_t e) {
+    cudaGetLastError();
+    return std::string(what) + " failed: " + cudaGetErrorString(e);
+}
+
+// k = min(members, n, max(1, total / min_share)); messages sorted by length (longest first, stable) and dealt over
+// 0..k-1 in boustrophedon order -- the same deal as sharding.shard_assignment(lengths, k).
+int split_owner(const uint64_t* len, uint64_t n, int nmembers, uint64_t min_share, uint32_t* owner) {
+    if (min_share == 0) min_share = B200H_GROUP_MIN_SHARE;
+    uint64_t total = 0;
+    for (uint64_t i = 0; i < n; ++i) total += len[i];
+    const uint64_t k = std::min<uint64_t>({(uint64_t)std::max(nmembers, 0), n, std::max<uint64_t>(1, total / min_share)});
+    if (k == 0) return 0;
+    std::vector<uint64_t> order(n);
+    std::iota(order.begin(), order.end(), uint64_t(0));
+    std::stable_sort(order.begin(), order.end(), [&](uint64_t a, uint64_t b) { return len[a] > len[b]; });
+    for (uint64_t p = 0; p < n; ++p) {
+        const uint64_t lap = p / k, col = p % k;
+        owner[order[p]] = (uint32_t)((lap & 1) ? k - 1 - col : col);
+    }
+    return (int)k;
+}
+
+int group_fail(b200h_group* g, int code, const std::string& msg) {
+    std::lock_guard<std::mutex> lk(g->mu);
+    g->err = msg;
+    return code;
+}
+
+std::string member_prefix(b200h_group* g, int j) {
+    return "member " + std::to_string(j) + " (cuda:" + std::to_string(g->members[j]->device) + "): ";
+}
+
+// Host or device memory?  Device columns must all sit on one device.
+int classify_outputs(b200h_group* g, Columns& c) {
+    for (int k = 0; k < 3; ++k) {
+        if (!c.out[k]) continue;
+        cudaPointerAttributes at;
+        if (cudaPointerGetAttributes(&at, c.out[k]) != cudaSuccess) {
+            cudaGetLastError();
+            continue;  // plain pageable host memory
+        }
+        if (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) continue;
+        if (c.table_device >= 0 && c.table_device != at.device)
+            return group_fail(g, B200H_E_INVALID, "device outputs must all be on one device (got cuda:" +
+                                                      std::to_string(c.table_device) + " and cuda:" +
+                                                      std::to_string(at.device) + ")");
+        c.on_device[k] = true;
+        c.table_device = at.device;
+    }
+    return 0;
+}
+
+int ensure_scratch(DevScratch& s, int device, size_t bytes, std::string* err) {
+    if (s.device == device && s.cap >= bytes) return 0;
+    if (s.p) {
+        cudaSetDevice(s.device);
+        cudaFree(s.p);
+        s.p = nullptr;
+        s.cap = 0;
+    }
+    s.device = device;
+    const size_t want = std::max<size_t>(bytes, size_t(1) << 20);
+    cudaError_t e = cudaSetDevice(device);
+    if (e == cudaSuccess) e = cudaMalloc((void**)&s.p, want);
+    if (e != cudaSuccess) {
+        *err = cuda_msg("cudaMalloc (group scatter buffer)", e);
+        s.p = nullptr;
+        return e == cudaErrorMemoryAllocation ? B200H_E_NOMEM : B200H_E_CUDA;
+    }
+    s.cap = want;
+    return 0;
+}
+
+// May the member's device write into memory on `table`?  Peer access is enabled for this process's contexts only.
+bool peer_ok(Member& m, int table) {
+    if (table == m.device) return true;
+    if ((int)m.peer.size() <= table) m.peer.resize(table + 1, -1);
+    if (m.peer[table] < 0) {
+        int can = 0;
+        m.peer[table] = 0;
+        if (cudaDeviceCanAccessPeer(&can, m.device, table) == cudaSuccess && can) {
+            cudaSetDevice(m.device);
+            const cudaError_t e = cudaDeviceEnablePeerAccess(table, 0);
+            m.peer[table] = (e == cudaSuccess || e == cudaErrorPeerAccessAlreadyEnabled) ? 1 : 0;
+        }
+        cudaGetLastError();
+    }
+    return m.peer[table] == 1;
+}
+
+int launch_scatter(const uint8_t* src, const uint64_t* idx, uint64_t rows, uint32_t width, uint8_t* dst, cudaStream_t st) {
+    const uint64_t total = rows * width;
+    const unsigned blocks = (unsigned)std::min<uint64_t>((total + 255) / 256, 148 * 16);
+    scatter_rows_kernel<<<blocks, 256, 0, st>>>(src, idx, rows, width, dst);
+    return 1;
+}
+
+#define GROUP_CU(call)                                   \
+    do {                                                 \
+        cudaError_t e__ = (call);                        \
+        if (e__ != cudaSuccess) {                        \
+            s.err = cuda_msg(#call, e__);                \
+            return B200H_E_CUDA;                         \
+        }                                                \
+    } while (0)
+
+// The device columns of a finished share (in m.share, column k at col_at[k], row indices at idx_at) into the table.
+int scatter_device(Member& m, const Columns& c, Share& s, const size_t* col_at, size_t idx_at, size_t used) {
+    const uint64_t rows = s.idx.size();
+    if (!m.st) {
+        GROUP_CU(cudaSetDevice(m.device));
+        GROUP_CU(cudaStreamCreateWithFlags(&m.st, cudaStreamNonBlocking));
+    }
+    const uint8_t* from = m.share.p;
+    int dev = m.device;
+    cudaStream_t st = m.st;
+    if (!peer_ok(m, c.table_device)) {
+        // no peer access: move the share (columns and indices) to the table device and scatter there
+        if (int rc = ensure_scratch(m.staged, c.table_device, used, &s.err)) return rc;
+        if (m.st_table && m.staged.device != c.table_device) {
+            cudaStreamDestroy(m.st_table);
+            m.st_table = nullptr;
+        }
+        GROUP_CU(cudaSetDevice(c.table_device));
+        if (!m.st_table) GROUP_CU(cudaStreamCreateWithFlags(&m.st_table, cudaStreamNonBlocking));
+        GROUP_CU(cudaMemcpyPeerAsync(m.staged.p, c.table_device, m.share.p, m.device, idx_at, m.st_table));
+        GROUP_CU(cudaMemcpyAsync(m.staged.p + idx_at, s.idx.data(), rows * 8, cudaMemcpyHostToDevice, m.st_table));
+        from = m.staged.p;
+        dev = c.table_device;
+        st = m.st_table;
+    } else {
+        GROUP_CU(cudaSetDevice(dev));
+        GROUP_CU(cudaMemcpyAsync(m.share.p + idx_at, s.idx.data(), rows * 8, cudaMemcpyHostToDevice, st));
+    }
+    for (int k = 0; k < 3; ++k)
+        if (c.out[k] && c.on_device[k])
+            launch_scatter(from + col_at[k], (const uint64_t*)(from + idx_at), rows, c.width[k], c.out[k], st);
+    GROUP_CU(cudaGetLastError());
+    GROUP_CU(cudaStreamSynchronize(st));
+    return 0;
+}
+
+// What one worker does with its member's share: hash it into share-sized outputs, scatter the rows.
+void run_share(b200h_group* g, int j, const uint8_t* base, const char* const* paths, uint32_t flags, const Columns& c,
+               Share& s) {
+    const auto t0 = Clock::now();
+    Member& m = *g->members[j];
+    const uint64_t rows = s.idx.size();
+    std::vector<uint8_t> host[3];
+    uint8_t* to[3] = {nullptr, nullptr, nullptr};
+    size_t col_at[3] = {0, 0, 0}, used = 0;
+    for (int k = 0; k < 3; ++k) {
+        if (!c.out[k]) continue;
+        if (c.on_device[k]) {
+            col_at[k] = used;
+            used += (rows * c.width[k] + 255) & ~size_t(255);
+        } else {
+            host[k].resize(rows * c.width[k]);
+            to[k] = host[k].data();
+        }
+    }
+    const size_t idx_at = used;
+    if (used) {
+        used += rows * 8;
+        if ((s.rc = ensure_scratch(m.share, m.device, used, &s.err))) return;
+        for (int k = 0; k < 3; ++k)
+            if (c.out[k] && c.on_device[k]) to[k] = m.share.p + col_at[k];
+    }
+    s.rc = b200h::hash_share(m.ctx, base, s.off.data(), s.len.data(), rows, flags, to[0], to[1], (uint64_t*)to[2], paths,
+                             paths ? s.file_of.data() : nullptr, &s.staged);
+    if (s.rc) {
+        s.err = b200h_last_error(m.ctx);
+    } else {
+        for (int k = 0; k < 3; ++k) {
+            if (!c.out[k] || c.on_device[k]) continue;
+            const uint32_t w = c.width[k];
+            for (uint64_t r = 0; r < rows; ++r) memcpy(c.out[k] + s.idx[r] * w, host[k].data() + r * w, w);
+        }
+        if (used) s.rc = scatter_device(m, c, s, col_at, idx_at, used);
+    }
+    s.ms = ms_since(t0);
+}
+
+void record_split(b200h_group* g, const std::vector<Share>& shares) {
+    const size_t nm = g->members.size();
+    g->last_messages.assign(nm, 0);
+    g->last_bytes.assign(nm, 0);
+    g->last_staged.assign(nm, 0);
+    g->last_ms.assign(nm, 0.0);
+    for (size_t j = 0; j < shares.size(); ++j) {
+        g->last_messages[j] = shares[j].idx.size();
+        g->last_bytes[j] = shares[j].bytes;
+        g->last_staged[j] = shares[j].staged;
+        g->last_ms[j] = shares[j].ms;
+    }
+}
+
+// Deal messages (off, len, file_of) over the members, run every share on its member's worker, wait for all of them.
+int run_split(b200h_group* g, const uint8_t* base, const char* const* paths, const uint64_t* off, const uint64_t* len,
+              const uint64_t* file_of, uint64_t n, uint32_t flags, const Columns& c, int k, const uint32_t* owner) {
+    std::vector<Share> shares(k);
+    for (uint64_t i = 0; i < n; ++i) {
+        Share& s = shares[owner[i]];
+        s.idx.push_back(i);
+        s.off.push_back(off[i]);
+        s.len.push_back(len[i]);
+        if (file_of) s.file_of.push_back(file_of[i]);
+        s.bytes += len[i];
+    }
+    std::mutex dm;
+    std::condition_variable dcv;
+    int left = k;
+    for (int j = 0; j < k; ++j)
+        g->members[j]->worker->post([&, j] {
+            run_share(g, j, base, paths, flags, c, shares[j]);
+            std::lock_guard<std::mutex> lk(dm);  // notify under the lock: the waiter's cv lives on its stack
+            --left;
+            dcv.notify_one();
+        });
+    {
+        std::unique_lock<std::mutex> lk(dm);
+        dcv.wait(lk, [&] { return left == 0; });
+    }
+    std::lock_guard<std::mutex> lk(g->mu);
+    record_split(g, shares);
+    for (int j = 0; j < k; ++j)
+        if (shares[j].rc) {
+            g->err = member_prefix(g, j) + shares[j].err;
+            return shares[j].rc;
+        }
+    return 0;
+}
+
+// k <= 1: the home member's own entry point, exactly.
+template <typename F>
+int run_home(b200h_group* g, uint64_t n, const uint64_t* len, F call) {
+    b200h_ctx* home = g->members[0]->ctx;
+    const auto t0 = Clock::now();
+    const uint64_t staged0 = b200h::staged_bytes(home);
+    const int rc = call(home);
+    std::vector<Share> one(1);
+    one[0].idx.resize(n);
+    for (uint64_t i = 0; i < n; ++i) one[0].bytes += len[i];
+    one[0].staged = b200h::staged_bytes(home) - staged0;
+    one[0].ms = ms_since(t0);
+    std::lock_guard<std::mutex> lk(g->mu);
+    record_split(g, one);
+    if (rc) g->err = member_prefix(g, 0) + b200h_last_error(home);
+    return rc;
+}
+
+}  // namespace
+
+extern "C" {
+
+int b200h_group_create(const int* devices, int ndevices, size_t pinned_bytes, size_t device_bytes,
+                       uint64_t min_share_bytes, b200h_group** out) {
+    if (!out) {
+        g_group_create_error = "out is NULL";
+        return B200H_E_INVALID;
+    }
+    *out = nullptr;
+    if (!devices || ndevices < 1) {
+        g_group_create_error = "a group needs at least one device";
+        return B200H_E_INVALID;
+    }
+    b200h_group* g = new (std::nothrow) b200h_group();
+    if (!g) {
+        g_group_create_error = "out of host memory";
+        return B200H_E_NOMEM;
+    }
+    g->min_share = min_share_bytes ? min_share_bytes : B200H_GROUP_MIN_SHARE;
+    for (int i = 0; i < ndevices; ++i) {
+        b200h_ctx* ctx = nullptr;
+        const int rc = b200h::create_member(devices[i], pinned_bytes, device_bytes, devices, ndevices, &ctx);
+        if (rc) {
+            g_group_create_error = "member " + std::to_string(i) + " (cuda:" + std::to_string(devices[i]) +
+                                   "): " + b200h_last_error(nullptr);
+            b200h_group_destroy(g);
+            return rc;
+        }
+        std::unique_ptr<Member> m(new Member());
+        m->ctx = ctx;
+        m->device = devices[i];
+        m->worker.reset(new Worker());
+        g->members.push_back(std::move(m));
+    }
+    *out = g;
+    return 0;
+}
+
+void b200h_group_destroy(b200h_group* g) {
+    if (!g) return;
+    for (auto& m : g->members) m->worker.reset();  // joins: no share is in flight after this
+    for (auto& m : g->members) {
+        for (DevScratch* s : {&m->share, &m->staged})
+            if (s->p) {
+                cudaSetDevice(s->device);
+                cudaFree(s->p);
+            }
+        if (m->st) {
+            cudaSetDevice(m->device);
+            cudaStreamDestroy(m->st);
+        }
+        if (m->st_table) {
+            cudaSetDevice(m->staged.device);
+            cudaStreamDestroy(m->st_table);
+        }
+        b200h_destroy(m->ctx);
+    }
+    cudaGetLastError();
+    delete g;
+}
+
+const char* b200h_group_last_error(b200h_group* g) { return g ? g->err.c_str() : g_group_create_error.c_str(); }
+
+int b200h_group_size(b200h_group* g) { return g ? (int)g->members.size() : 0; }
+
+b200h_ctx* b200h_group_member(b200h_group* g, int i) {
+    if (!g || i < 0 || i >= (int)g->members.size()) return nullptr;
+    return g->members[i]->ctx;
+}
+
+int b200h_group_hash_batch_host(b200h_group* g, const uint8_t* base, const uint64_t* offsets, const uint64_t* lengths,
+                                uint64_t n, uint32_t flags, uint8_t* sha256_out, uint8_t* md5_out,
+                                uint64_t* trimmed_len_out) {
+    if (!g) return B200H_E_INVALID;
+    if (n && (!offsets || !lengths)) return group_fail(g, B200H_E_INVALID, "offsets/lengths must not be NULL");
+    if (!(flags & (B200H_SHA256 | B200H_MD5))) return group_fail(g, B200H_E_INVALID, "flags select neither SHA256 nor MD5");
+    std::vector<uint32_t> owner(n);
+    const int k = n ? split_owner(lengths, n, (int)g->members.size(), g->min_share, owner.data()) : 0;
+    if (k <= 1)
+        return run_home(g, n, lengths, [&](b200h_ctx* home) {
+            return b200h_hash_batch_host(home, base, offsets, lengths, n, flags, sha256_out, md5_out, trimmed_len_out);
+        });
+    const uint32_t wide = (flags & B200H_HEX_OUT) ? 2 : 1;
+    Columns c;
+    c.out[0] = (flags & B200H_SHA256) ? sha256_out : nullptr;
+    c.out[1] = (flags & B200H_MD5) ? md5_out : nullptr;
+    c.out[2] = (uint8_t*)trimmed_len_out;
+    c.width[0] = 32 * wide;
+    c.width[1] = 16 * wide;
+    if (int rc = classify_outputs(g, c)) return rc;
+    return run_split(g, base, nullptr, offsets, lengths, nullptr, n, flags, c, k, owner.data());
+}
+
+int b200h_group_hash_files(b200h_group* g, const char* const* paths, uint64_t n, const uint64_t* sizes,
+                           uint64_t part_len, uint32_t flags, uint8_t* sha256_out, uint8_t* md5_out,
+                           uint64_t* trimmed_len_out) {
+    if (!g) return B200H_E_INVALID;
+    if (n && (!paths || !sizes)) return group_fail(g, B200H_E_INVALID, "paths/sizes must not be NULL");
+    if (!(flags & (B200H_SHA256 | B200H_MD5))) return group_fail(g, B200H_E_INVALID, "flags select neither SHA256 nor MD5");
+    std::vector<uint64_t> off, len, file_of;
+    b200h::file_messages(sizes, n, part_len, off, len, file_of);
+    const uint64_t rows = off.size();
+    std::vector<uint32_t> owner(rows);
+    const int k = rows ? split_owner(len.data(), rows, (int)g->members.size(), g->min_share, owner.data()) : 0;
+    if (k <= 1)
+        return run_home(g, rows, len.data(), [&](b200h_ctx* home) {
+            return b200h_hash_files(home, paths, n, sizes, part_len, flags, sha256_out, md5_out, trimmed_len_out);
+        });
+    const uint32_t wide = (flags & B200H_HEX_OUT) ? 2 : 1;
+    Columns c;
+    c.out[0] = (flags & B200H_SHA256) ? sha256_out : nullptr;
+    c.out[1] = (flags & B200H_MD5) ? md5_out : nullptr;
+    c.out[2] = (uint8_t*)trimmed_len_out;
+    c.width[0] = 32 * wide;
+    c.width[1] = 16 * wide;
+    if (int rc = classify_outputs(g, c)) return rc;
+    return run_split(g, nullptr, paths, off.data(), len.data(), file_of.data(), rows, flags, c, k, owner.data());
+}
+
+int b200h_group_last_split(b200h_group* g, uint64_t* messages_out, uint64_t* bytes_out, uint64_t* staged_bytes_out,
+                           double* busy_ms_out) {
+    if (!g) return B200H_E_INVALID;
+    std::lock_guard<std::mutex> lk(g->mu);
+    const size_t nm = g->members.size();
+    for (size_t j = 0; j < nm; ++j) {
+        const bool have = j < g->last_messages.size();
+        if (messages_out) messages_out[j] = have ? g->last_messages[j] : 0;
+        if (bytes_out) bytes_out[j] = have ? g->last_bytes[j] : 0;
+        if (staged_bytes_out) staged_bytes_out[j] = have ? g->last_staged[j] : 0;
+        if (busy_ms_out) busy_ms_out[j] = have ? g->last_ms[j] : 0.0;
+    }
+    return 0;
+}
+
+int b200h_group_split_preview(const uint64_t* lengths, uint64_t n, int nmembers, uint64_t min_share_bytes,
+                              uint32_t* owner_out, int* members_used_out) {
+    if ((n && (!lengths || !owner_out)) || nmembers < 1) return B200H_E_INVALID;
+    const int k = n ? split_owner(lengths, n, nmembers, min_share_bytes, owner_out) : 0;
+    if (members_used_out) *members_used_out = k;
+    return 0;
+}
+
+}  // extern "C"
