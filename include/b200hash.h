@@ -114,6 +114,25 @@ int b200h_hash_fixed_parts(b200h_ctx* ctx, const uint8_t* base, uint64_t len, ui
                            uint8_t* sha256_out, uint8_t* md5_out, uint64_t* trimmed_len_out,
                            uint8_t etag_md5_out[16], uint64_t* nparts_out);
 
+/* ---- buffers already in HBM, split into parts ------------------------------------------------------ */
+
+/* The device-memory twin of b200h_hash_files(part_len): n buffers [d_bufs[i], +sizes[i]), each DEVICE memory on ctx's
+ * device (any alignment), are hashed where they are.
+ *   part_len == 0: one row per buffer (a zero-size buffer gives the empty-message digest);
+ *   part_len  > 0: ceil(size/part_len) rows per buffer, flattened buffer-major (a zero-size buffer gives no rows);
+ *                  with B200H_TRIM_ZEROS these are the volumefs2 blocks of a tensor's raw bytes.
+ * Flags as for the host entry points (B200H_SHA256, B200H_MD5, B200H_TRIM_ZEROS, B200H_HEX_OUT).  etag_md5_out (n*16,
+ * may be NULL; requires B200H_MD5): row i = MD5 over the concatenated raw part MD5s of buffer i, the multipart ETag of
+ * b200h_hash_fixed_parts, computed on the device for every buffer in one more launch.  Outputs may be host or device
+ * memory (cudaMemcpyDefault); the call returns when they are written.  The part table is built on the host and copied
+ * once; nothing is read back except the planner's count when B200H_TRIM_ZEROS is set (see b200h_hash_batch_device).
+ * A buffer that is not device memory on ctx's device is B200H_E_INVALID, last_error naming the buffer index and where
+ * it lives.  Replaces: t.cpu() + a scratch file + the per-block reads of _gather_blocks / the whole-file hashlib
+ * passes of _get_file_upload_spec for a tensor written to a Volume. */
+int b200h_hash_device_parts(b200h_ctx* ctx, const void* const* d_bufs, const uint64_t* sizes, uint64_t n,
+                            uint64_t part_len, uint32_t flags, uint8_t* sha256_out, uint8_t* md5_out,
+                            uint64_t* trimmed_len_out, uint8_t* etag_md5_out);
+
 /* ---- files (native reader pool; no Python I/O, no mmap) ------------------------------------------ */
 
 /* Sizes (and permission bits, may be NULL) of n regular files, stat'ed by the library's I/O threads.
@@ -204,6 +223,7 @@ int b200h_profile_read(b200h_ctx* ctx, double* hash_kernel_ms, uint64_t* hash_ke
  * b200h_group_hash_batch_host / _hash_files deal a batch over the members by bytes (b200h_group_split_preview), every
  * member hashes its share on its own thread at the same time, and the rows land at the caller's message indices.
  * Members on one NUMA node divide its CPUs between their packer and reader teams.  Group calls are thread-safe.
+ * b200h_group_hash_device_parts deals the parts of buffers already in HBM over the members on each buffer's device.
  * Everything else (stat_files, dedupe_*, hash_fixed_parts, streams, host_alloc, the *_device entry points) is not
  * split: call it on b200h_group_member(g, 0), the "home" member.  Its host_alloc memory is portable, so every member
  * DMAs it directly. */
@@ -232,6 +252,15 @@ int b200h_group_hash_batch_host(b200h_group* g, const uint8_t* base, const uint6
 int b200h_group_hash_files(b200h_group* g, const char* const* paths, uint64_t n, const uint64_t* sizes,
                            uint64_t part_len, uint32_t flags, uint8_t* sha256_out, uint8_t* md5_out,
                            uint64_t* trimmed_len_out);
+/* As b200h_hash_device_parts.  A buffer is only hashed by members on the device that holds it: the parts resident on
+ * device d are dealt over the members on d by the rule above, so {0, 0} splits one GPU's parts and {0, 1} hashes each
+ * GPU's buffers on that GPU.  Every member works on its own thread and the rows land at their global indices; ETags
+ * are computed after all MD5 rows are in place.  A buffer on a device with no member is B200H_E_INVALID ("buffer 3 is
+ * on cuda:5, which is not in the group"); the group stays usable.  When one member takes the whole batch this IS
+ * b200h_hash_device_parts on that member. */
+int b200h_group_hash_device_parts(b200h_group* g, const void* const* d_bufs, const uint64_t* sizes, uint64_t n,
+                                  uint64_t part_len, uint32_t flags, uint8_t* sha256_out, uint8_t* md5_out,
+                                  uint64_t* trimmed_len_out, uint8_t* etag_md5_out);
 /* What the last batch call did, per member (arrays of b200h_group_size entries, each may be NULL): messages, payload
  * bytes, bytes that went through the member's pinned staging ring (0 = DMAed straight from the caller's page-locked
  * memory) and wall milliseconds spent inside the member.  Members the batch did not use report zeros. */

@@ -35,6 +35,7 @@ ABI_SYMBOLS = (
     "b200h_stream_copy", "b200h_stream_copy_isa", "b200h_plan_preview", "b200h_pack_preview",
     "b200h_group_create", "b200h_group_destroy", "b200h_group_last_error", "b200h_group_size", "b200h_group_member",
     "b200h_group_hash_batch_host", "b200h_group_hash_files", "b200h_group_last_split", "b200h_group_split_preview",
+    "b200h_hash_device_parts", "b200h_group_hash_device_parts",
 )
 
 
@@ -44,7 +45,7 @@ class B200HashError(RuntimeError):
 
 def build_library(force: bool = False, verbose: bool = False) -> str:
     srcs = [os.path.join(CSRC, f) for f in ("b200hash_kernels.cu", "b200hash_dedupe.cu", "b200hash_api.cu",
-                                            "b200hash_group.cu", "b200hash_internal.h", "b200blob_host.cpp",
+                                            "b200hash_group.cu", "b200hash_device_parts.cu", "b200hash_internal.h", "b200blob_host.cpp",
                                             "b200pack_copy.cpp", "b200hash_kernels.cuh", "b200pack_team.h")]
     srcs += [os.path.join(os.path.dirname(_PKG), "include", h) for h in ("b200hash.h", "b200blob.h")]
     stale = not os.path.exists(LIB_PATH) or any(os.path.getmtime(s) > os.path.getmtime(LIB_PATH) for s in srcs)
@@ -155,6 +156,10 @@ def load_library() -> ctypes.CDLL:
         L.b200h_group_last_split.restype = i32
         L.b200h_group_split_preview.argtypes = [vp, u64, i32, u64, vp, ctypes.POINTER(i32)]
         L.b200h_group_split_preview.restype = i32
+        L.b200h_hash_device_parts.argtypes = [vp, vp, vp, u64, u64, u32, vp, vp, vp, vp]
+        L.b200h_hash_device_parts.restype = i32
+        L.b200h_group_hash_device_parts.argtypes = [vp, vp, vp, u64, u64, u32, vp, vp, vp, vp]
+        L.b200h_group_hash_device_parts.restype = i32
         _lib = L
         return L
 
@@ -380,6 +385,33 @@ class Context:
         assert got.value == nparts
         return sha, md5, trimmed, (etag.tobytes() if want_etag else None)
 
+    # -- buffers already in device memory, split into parts (b200h_hash_device_parts)
+    def hash_device_parts(self, ptrs, sizes, part_len: int, flags: int = SHA256 | MD5, want_etag: bool = False, *,
+                          out_sha: int = 0, out_md5: int = 0, out_trimmed: int = 0, out_etag: int = 0):
+        """ptrs: device addresses (e.g. CUDA tensors' data_ptr()) of n buffers on this context's device, sizes their
+        byte counts.  -> (sha[rows,32]|None, md5[rows,16]|None, trimmed[rows], etags[n,16]|None); rows = n (part_len 0)
+        or the buffer-major list of ceil(size/part_len) parts.  out_*: raw addresses (host or device memory) that
+        receive a column instead of a fresh numpy array; that element of the result is then None."""
+        p = np.ascontiguousarray(ptrs, dtype=np.uint64)
+        sz = np.ascontiguousarray(sizes, dtype=np.uint64)
+        n = int(p.size)
+        assert sz.size == n
+        rows = n if part_len == 0 else int(((sz + np.uint64(part_len - 1)) // np.uint64(part_len)).sum())
+        wide = 2 if flags & HEX_OUT else 1
+        sha = np.empty((rows, 32 * wide), np.uint8) if (flags & SHA256 and not out_sha) else None
+        md5 = np.empty((rows, 16 * wide), np.uint8) if (flags & MD5 and not out_md5) else None
+        trimmed = None if out_trimmed else np.empty(rows, np.uint64)
+        etag = np.empty((n, 16), np.uint8) if (want_etag and not out_etag) else None
+        self._device_parts(_np_ptr(p) if n else None, _np_ptr(sz) if n else None, n, part_len, flags,
+                           ctypes.c_void_p(out_sha) if out_sha else _np_ptr(sha),
+                           ctypes.c_void_p(out_md5) if out_md5 else _np_ptr(md5),
+                           ctypes.c_void_p(out_trimmed) if out_trimmed else _np_ptr(trimmed),
+                           ctypes.c_void_p(out_etag) if out_etag else _np_ptr(etag))
+        return sha, md5, trimmed, etag
+
+    def _device_parts(self, *args):
+        self._check(self._L.b200h_hash_device_parts(self._h, *args), "b200h_hash_device_parts")
+
     # -- files: stat + read + hash entirely inside the library (native reader threads, no mmap / Python I/O)
     @staticmethod
     def _c_paths(paths):
@@ -443,6 +475,7 @@ class Context:
 class DeviceGroup(Context):
     """One context per listed device, driven as one (include/b200hash.h, device groups).  ``hash_batch_host`` (and so
     ``hash_buffers``) and ``hash_files`` deal each batch over the members by bytes and hash the shares at the same time;
+    ``hash_device_parts`` deals the parts of device buffers over the members on each buffer's device;
     every other method runs on the home member (``devices[0]``), whose handle this object carries as a Context.
     ``devices=None`` means every visible device; a device may repeat.  ``min_share_bytes`` 0 = the library default."""
 
@@ -473,6 +506,10 @@ class DeviceGroup(Context):
 
     def _files(self, *args):
         self._gcheck(self._L.b200h_group_hash_files(self._g, *args), "b200h_group_hash_files")
+
+    def _device_parts(self, *args):
+        # every buffer is hashed by the members on the device that holds it
+        self._gcheck(self._L.b200h_group_hash_device_parts(self._g, *args), "b200h_group_hash_device_parts")
 
     def close(self):
         if getattr(self, "_g", None):

@@ -117,5 +117,36 @@ def hash_table_tensors(tensors: Sequence, *, sha256: bool = True, md5: bool = Tr
     return d_sha, d_md5
 
 
-__all__ = ["DigestTable", "hash_table_host", "hash_table_buffers", "hash_table_tensors", "Context", "default_context",
-           "_lib"]
+def ready_event(tensor):
+    """A CUDA event recorded on ``tensor``'s current torch stream: once it has completed, every write queued so far on
+    that stream is visible to the library's own streams.  Record it when a tensor is queued, wait on it before
+    hashing -- a wait on one event, not a device-wide synchronisation."""
+    import torch
+
+    ev = torch.cuda.Event()
+    ev.record(torch.cuda.current_stream(tensor.device))
+    return ev
+
+
+def hash_blocks_tensors(tensors: Sequence, part_len: int, *, sha256: bool = True, md5: bool = False,
+                        trim_zeros: bool = False, ctx: Context | None = None, ready: Sequence | None = None) -> DigestTable:
+    """Digest the raw bytes (``numel * element_size`` from ``data_ptr()``) of contiguous CUDA tensors of any dtype where
+    they are, split into ``part_len``-byte parts (``part_len`` 0: one row per tensor): ``b200h_hash_device_parts``.
+    Rows are tensor-major, ceil(nbytes / part_len) per tensor; with ``trim_zeros`` these are the volumefs2 blocks of the
+    tensor's bytes.  ``ready``: events from ``ready_event`` recorded when the tensors were queued (default: recorded
+    now); the call waits on them, so work already queued on each tensor's stream is part of what is hashed.  A device
+    group hashes every tensor on the members on its device."""
+    ctx = ctx or get_context()
+    for t in tensors:
+        if not (getattr(t, "is_cuda", False) and t.is_contiguous()):
+            raise ValueError("hash_blocks_tensors needs contiguous CUDA tensors")
+    for ev in (ready if ready is not None else [ready_event(t) for t in tensors]):
+        ev.synchronize()
+    flags = (SHA256 if sha256 else 0) | (MD5 if md5 else 0) | (TRIM_ZEROS if trim_zeros else 0)
+    s, m, t, _ = ctx.hash_device_parts([x.data_ptr() for x in tensors], [x.numel() * x.element_size() for x in tensors],
+                                       part_len, flags)
+    return DigestTable(s, m, t)
+
+
+__all__ = ["DigestTable", "hash_table_host", "hash_table_buffers", "hash_table_tensors", "hash_blocks_tensors",
+           "ready_event", "Context", "default_context", "_lib"]

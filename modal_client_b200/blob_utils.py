@@ -24,9 +24,11 @@ import asyncio
 import dataclasses
 import functools
 import gc
+import io
 import mmap
 import os
 import platform
+import threading
 import time
 from collections.abc import Callable, Sequence
 from contextlib import AbstractContextManager, asynccontextmanager, contextmanager
@@ -217,10 +219,14 @@ async def perform_multipart_upload(
     byte_budget: _ByteBudget | None = None,
 ) -> None:
     # 1. hash every part on the GPU before sending anything
-    start_pos = data_file.tell() if isinstance(data_file, BytesIO) else 0
-    part_md5, expected_etag = await asyncio.to_thread(
-        _with_view, data_file,
-        lambda whole: multipart_part_digests(whole[start_pos : start_pos + content_length], max_part_size))
+    on_device = isinstance(data_file, DeviceBufferReader)
+    start_pos = data_file.tell() if isinstance(data_file, (BytesIO, DeviceBufferReader)) else 0
+    if on_device:  # a tensor's bytes: the parts are hashed where they are, nothing is copied to the host for it
+        part_md5, expected_etag = await asyncio.to_thread(data_file.part_digests, start_pos, content_length, max_part_size)
+    else:
+        part_md5, expected_etag = await asyncio.to_thread(
+            _with_view, data_file,
+            lambda whole: multipart_part_digests(whole[start_pos : start_pos + content_length], max_part_size))
     if len(part_md5) > len(part_urls):
         raise ExecutionError(f"{len(part_md5)} parts but only {len(part_urls)} part URLs")
 
@@ -228,6 +234,10 @@ async def perform_multipart_upload(
     if isinstance(data_file, BytesIO):
         view = data_file.getbuffer()
         readers: list[BinaryIO] = [BytesIO(view) for _ in part_urls]
+        for rdr in readers:
+            rdr.seek(start_pos)
+    elif on_device:
+        readers = [data_file.clone() for _ in part_urls]
         for rdr in readers:
             rdr.seek(start_pos)
     else:
@@ -886,6 +896,204 @@ async def file_upload_specs2(
         return out
 
     return await asyncio.to_thread(run)
+
+
+# ------------------------------------------------------------------------- tensors already in HBM
+
+
+class _ByteCounter:
+    def __init__(self):
+        self._lock = threading.Lock()
+        self.total = 0
+
+    def add(self, n: int) -> None:
+        with self._lock:
+            self.total += n
+
+
+class DeviceBufferReader(io.RawIOBase):
+    """Read-only, seekable binary file object over the raw bytes of a contiguous tensor (``numel * element_size`` from
+    ``data_ptr()``).  ``read(n)`` copies only that range to the host, ``stage_bytes`` at a time through a small pinned
+    buffer, so host memory is bounded by the reads in flight (the PUTs), never by the tensor size.  ``clone()`` gives
+    an independent reader (own position and staging buffer) over the same bytes; every clone adds to the same
+    ``bytes_to_host`` count, which is what crossed PCIe.  Used as a spec's ``source()``, it lets ``_put_missing_blocks``,
+    ``BytesIOSegmentPayload`` and ``blob_upload_file`` run unchanged.
+
+    The reader waits, before its first copy, on a CUDA event recorded on the tensor's current stream when the reader
+    was made (``ready``): work queued before that is visible, later writes to the tensor are not allowed until the
+    upload is done.  A CPU tensor is read with plain copies (host-backed reader, for host-side tests)."""
+
+    def __init__(self, tensor, *, stage_bytes: int = 4 << 20, _root: "DeviceBufferReader | None" = None):
+        super().__init__()
+        if _root is None:
+            if not tensor.is_contiguous():
+                raise ValueError("DeviceBufferReader needs a contiguous tensor")
+            self.tensor = tensor
+            self.nbytes = tensor.numel() * tensor.element_size()
+            self._flat = tensor.reshape(-1).view(_torch().uint8) if self.nbytes else None
+            self._counter = _ByteCounter()
+            self._ready = None
+            if tensor.is_cuda:
+                from .batch import ready_event
+
+                self._ready = ready_event(tensor)
+        else:
+            self.tensor, self.nbytes, self._flat = _root.tensor, _root.nbytes, _root._flat
+            self._counter, self._ready = _root._counter, _root._ready
+        self._stage_bytes = stage_bytes
+        self._pos = 0
+        self._pin = self._pin_np = self._stream = None
+
+    # ---- what the hash and upload layers ask -----------------------------------------------------------------
+    @property
+    def data_ptr(self) -> int:
+        return self.tensor.data_ptr()
+
+    @property
+    def device(self):
+        return self.tensor.device
+
+    @property
+    def bytes_to_host(self) -> int:
+        """Bytes this reader and its clones have copied to the host so far."""
+        return self._counter.total
+
+    def wait_ready(self) -> None:
+        """Block until the work queued on the tensor's stream before the reader was made has finished."""
+        if self._ready is not None:
+            self._ready.synchronize()
+
+    def clone(self) -> "DeviceBufferReader":
+        return DeviceBufferReader(None, stage_bytes=self._stage_bytes, _root=self)
+
+    def part_digests(self, start: int, length: int, part_length: int) -> tuple[list[bytes], str]:
+        """``multipart_part_digests`` of bytes [start, start + length), hashed on the device where they are: the part
+        MD5s and the multipart ETag from one ``b200h_hash_device_parts(part_length, MD5)`` call."""
+        self.wait_ready()
+        _, md5, _, etag = get_context().hash_device_parts([self.data_ptr + start], [length], part_length, _lib.MD5,
+                                                          want_etag=True)
+        return [md5[i].tobytes() for i in range(len(md5))], f"{etag[0].tobytes().hex()}-{len(md5)}"
+
+    # ---- io.RawIOBase ------------------------------------------------------------------------------------------
+    def readable(self) -> bool:
+        return True
+
+    def seekable(self) -> bool:
+        return True
+
+    def tell(self) -> int:
+        return self._pos
+
+    def seek(self, offset: int, whence: int = os.SEEK_SET) -> int:
+        base = {os.SEEK_SET: 0, os.SEEK_CUR: self._pos, os.SEEK_END: self.nbytes}[whence]
+        if base + offset < 0:
+            raise ValueError("negative seek position")
+        self._pos = base + offset
+        return self._pos
+
+    def read(self, size: int = -1) -> bytes:
+        n = max(0, self.nbytes - self._pos) if size is None or size < 0 else size
+        buf = bytearray(min(n, max(0, self.nbytes - self._pos)))
+        got = self.readinto(buf)
+        return bytes(buf) if got == len(buf) else bytes(buf[:got])
+
+    def readinto(self, b) -> int:
+        dst = np.frombuffer(memoryview(b).cast("B"), np.uint8)
+        n = max(0, min(dst.size, self.nbytes - self._pos))
+        if n == 0:
+            return 0
+        self._copy(self._pos, dst[:n])
+        self._pos += n
+        self._counter.add(n)
+        return n
+
+    def close(self) -> None:
+        self._pin = self._pin_np = self._stream = None
+        super().close()
+
+    def _copy(self, at: int, dst: np.ndarray) -> None:
+        src = self._flat[at : at + dst.size]
+        if not src.is_cuda:
+            dst[:] = src.numpy()
+            return
+        torch = _torch()
+        self.wait_ready()
+        if self._pin is None:
+            self._pin = torch.empty(min(self._stage_bytes, self.nbytes), dtype=torch.uint8, pin_memory=True)
+            self._pin_np = self._pin.numpy()
+            self._stream = torch.cuda.Stream(device=src.device)
+        step = self._pin.numel()
+        with torch.cuda.stream(self._stream):
+            for o in range(0, dst.size, step):
+                k = min(step, dst.size - o)
+                self._pin[:k].copy_(src[o : o + k], non_blocking=True)
+                self._stream.synchronize()
+                dst[o : o + k] = self._pin_np[:k]
+
+
+def _torch():
+    import torch
+
+    return torch
+
+
+def _reader_digests(readers: Sequence[DeviceBufferReader], part_len: int, flags: int, want_etag: bool = False):
+    """One ``hash_device_parts`` call over the bytes of every reader's tensor, once the work queued on each tensor's
+    stream has finished."""
+    for r in readers:
+        r.wait_ready()
+    return get_context().hash_device_parts([r.data_ptr for r in readers], [r.nbytes for r in readers], part_len, flags,
+                                           want_etag)
+
+
+def tensor_upload_specs(items: Sequence[tuple[DeviceBufferReader, PurePosixPath | str, int]]) -> list[FileUploadSpec]:
+    """``FileUploadSpec`` (volumefs1) for tensors queued with ``put_tensor``: whole-buffer SHA-256 + MD5 of each tensor's
+    bytes on the device (``hash_device_parts`` with part_len 0), the size classes of ``_size_class``.  Each digest of a
+    whole buffer is ONE serial chain on the chain kernel, about 71 MB/s (DESIGN §5.4): roughly 15 s for 1 GiB.  The
+    multipart part MD5s are computed later on the device as well (``perform_multipart_upload``)."""
+    if not items:
+        return []
+    readers = [r for r, _, _ in items]
+    sizes = [r.nbytes for r in readers]
+    classes = [_size_class(s) for s in sizes]
+    sha_hex, md5_hex = [""] * len(items), [_MD5_PLACEHOLDER] * len(items)
+    for want_md5 in (True, False):
+        idx = [i for i, c in enumerate(classes) if c[1] == want_md5]
+        if not idx:
+            continue
+        sha, md5, _, _ = _reader_digests([readers[i] for i in idx], 0, _lib.SHA256 | (_lib.MD5 if want_md5 else 0))
+        for row, i in enumerate(idx):
+            sha_hex[i] = sha[row].tobytes().hex()
+            if want_md5:
+                md5_hex[i] = md5[row].tobytes().hex()
+    return [
+        FileUploadSpec(source=r.clone, source_description=f"<tensor {tuple(r.tensor.shape)} {r.tensor.dtype}>",
+                       source_is_path=False, mount_filename=PurePosixPath(remote).as_posix(), use_blob=classes[i][0],
+                       sha256_hex=sha_hex[i], md5_hex=md5_hex[i], mode=mode & 0o7777, size=sizes[i])
+        for i, (r, remote, mode) in enumerate(items)
+    ]
+
+
+def tensor_upload_specs2(items: Sequence[tuple[DeviceBufferReader, PurePosixPath | str, int]]) -> list[FileUploadSpec2]:
+    """``FileUploadSpec2`` (volumefs2) for tensors queued with ``put_tensor``: every 8 MiB block of every tensor in ONE
+    ``hash_device_parts(BLOCK_SIZE, SHA256 | TRIM_ZEROS)`` call, the blocks exactly as ``file_upload_specs2`` builds
+    them.  Only the trimmed bytes of the blocks the server reports missing are ever copied to the host."""
+    if not items:
+        return []
+    readers = [r for r, _, _ in items]
+    bs = BLOCK_SIZE
+    sha, _, trimmed, _ = _reader_digests(readers, bs, _lib.SHA256 | _lib.TRIM_ZEROS)
+    trimmed_l, sha_raw = trimmed.tolist(), sha.tobytes()
+    out, row = [], 0
+    for r, remote, mode in items:
+        blocks = []
+        for start in range(0, r.nbytes, bs):
+            blocks.append(FileUploadBlock(start, start + trimmed_l[row], sha_raw[32 * row : 32 * row + 32]))
+            row += 1
+        out.append(FileUploadSpec2(source=r.clone, source_description=f"<tensor {tuple(r.tensor.shape)} {r.tensor.dtype}>",
+                                   path=PurePosixPath(remote).as_posix(), blocks=blocks, mode=mode & 0o7777,
+                                   size=r.nbytes))
+    return out
 
 
 def use_md5(url: str) -> bool:

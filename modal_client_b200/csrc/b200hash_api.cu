@@ -1037,6 +1037,98 @@ int b200h::hash_share(b200h_ctx* ctx, const uint8_t* base, const uint64_t* off, 
     return rc;
 }
 
+int b200h::ctx_device(b200h_ctx* ctx) { return ctx->device; }
+
+int b200h::ctx_fail(b200h_ctx* ctx, int code, const std::string& msg) {
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    return fail(ctx, code, msg);
+}
+
+int b200h::hash_device_rows(b200h_ctx* ctx, const uint64_t* addr, const uint64_t* len, uint64_t rows, uint32_t flags,
+                            uint8_t* sha_out, uint8_t* md5_out, uint64_t* trim_out, const uint64_t* row_of, uint64_t n,
+                            uint8_t* etag_out) {
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    flags &= kPublicFlags;
+    if (!(flags & (B200H_SHA256 | B200H_MD5))) return fail(ctx, B200H_E_INVALID, "flags select neither SHA256 nor MD5");
+    if (etag_out && !(flags & B200H_MD5)) return fail(ctx, B200H_E_INVALID, "etag requires B200H_MD5");
+    const uint64_t ne = etag_out ? n : 0;
+    if (rows == 0 && ne == 0) return 0;
+    CU_TRY(ctx, cudaSetDevice(ctx->device));
+    // One pinned table -- addresses | lengths | ETag segment offsets | ETag segment lengths -- and one copy of it.
+    // A zero-length row reads nothing; it is pointed at library scratch so that no kernel ever sees a stray address.
+    if (int rc = ensure_meta(ctx, 2 * rows + 2 * ne)) return rc;
+    if (int rc = ensure_dev(ctx, ctx->d_small, 256)) return rc;
+    uint64_t* h = ctx->h_meta;
+    for (uint64_t i = 0; i < rows; ++i) {
+        h[i] = len[i] ? addr[i] : (uint64_t)(uintptr_t)ctx->d_small.p;
+        h[rows + i] = len[i];
+    }
+    for (uint64_t b = 0; b < ne; ++b) {
+        h[2 * rows + b] = 16 * row_of[b];
+        h[2 * rows + ne + b] = 16 * (row_of[b + 1] - row_of[b]);
+    }
+    const size_t table_bytes = (2 * rows + 2 * ne) * sizeof(uint64_t);
+    if (int rc = ensure_dev(ctx, ctx->d_off, table_bytes)) return rc;
+    if (int rc = ensure_dev(ctx, ctx->d_trim, rows * sizeof(uint64_t) + 8)) return rc;
+    if (flags & B200H_SHA256)
+        if (int rc = ensure_dev(ctx, ctx->d_sha, rows * 32 + 32)) return rc;
+    if (flags & B200H_MD5)
+        if (int rc = ensure_dev(ctx, ctx->d_md5, rows * 16 + 16)) return rc;
+    // d_hex: hex SHA-256 rows | hex MD5 rows | ETags (16-byte aligned: rows * 96)
+    if (int rc = ensure_dev(ctx, ctx->d_hex, rows * 96 + ne * 16 + 64)) return rc;
+    uint64_t* d_tab = (uint64_t*)ctx->d_off.p;
+    uint64_t* d_trim = (uint64_t*)ctx->d_trim.p;
+    uint8_t* d_sha = (flags & B200H_SHA256) ? (uint8_t*)ctx->d_sha.p : nullptr;
+    uint8_t* d_md5 = (flags & B200H_MD5) ? (uint8_t*)ctx->d_md5.p : nullptr;
+    uint8_t* hex_sha = (uint8_t*)ctx->d_hex.p;
+    uint8_t* hex_md5 = hex_sha + rows * 64;
+    uint8_t* d_etag = hex_sha + rows * 96;
+    CU_TRY(ctx, cudaMemcpyAsync(d_tab, h, table_bytes, cudaMemcpyHostToDevice, ctx->s_comp));
+    // the lengths are known here: outliers are routed without a read-back (B200H_TRIM_ZEROS still needs its one)
+    if (rows)
+        if (int rc = enqueue_device_batch(ctx, nullptr, d_tab, d_tab + rows, rows, flags, d_sha, d_md5, d_trim, nullptr,
+                                          ctx->s_comp, len))
+            return rc;
+    if (ne)
+        // every buffer's ETag in one batch: message b = its segment of the raw MD5 table (blob_utils.py:216-219)
+        if (int rc = enqueue_device_batch(ctx, d_md5, d_tab + 2 * rows, d_tab + 2 * rows + ne, ne, B200H_MD5, nullptr,
+                                          d_etag, nullptr, nullptr, ctx->s_comp, h + 2 * rows + ne))
+            return rc;
+    if (flags & B200H_HEX_OUT) {
+        if (sha_out && d_sha && rows) {
+            ctx->launches += launch_hex_rows(d_sha, rows * 32, hex_sha, ctx->s_comp);
+            CU_TRY(ctx, cudaMemcpyAsync(sha_out, hex_sha, rows * 64, cudaMemcpyDefault, ctx->s_comp));
+        }
+        if (md5_out && d_md5 && rows) {
+            ctx->launches += launch_hex_rows(d_md5, rows * 16, hex_md5, ctx->s_comp);
+            CU_TRY(ctx, cudaMemcpyAsync(md5_out, hex_md5, rows * 32, cudaMemcpyDefault, ctx->s_comp));
+        }
+        CU_TRY(ctx, cudaGetLastError());
+    } else if (rows) {
+        if (sha_out && d_sha) CU_TRY(ctx, cudaMemcpyAsync(sha_out, d_sha, rows * 32, cudaMemcpyDefault, ctx->s_comp));
+        if (md5_out && d_md5) CU_TRY(ctx, cudaMemcpyAsync(md5_out, d_md5, rows * 16, cudaMemcpyDefault, ctx->s_comp));
+    }
+    if (trim_out && rows) CU_TRY(ctx, cudaMemcpyAsync(trim_out, d_trim, rows * sizeof(uint64_t), cudaMemcpyDefault, ctx->s_comp));
+    if (ne) CU_TRY(ctx, cudaMemcpyAsync(etag_out, d_etag, ne * 16, cudaMemcpyDefault, ctx->s_comp));
+    CU_TRY(ctx, cudaStreamSynchronize(ctx->s_comp));
+    return 0;
+}
+
+int b200h::hex_rows_from_host(b200h_ctx* ctx, const uint8_t* raw, uint64_t nbytes, uint8_t* out) {
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if (!nbytes) return 0;
+    CU_TRY(ctx, cudaSetDevice(ctx->device));
+    const uint64_t at = (nbytes + 255) & ~uint64_t(255);
+    if (int rc = ensure_dev(ctx, ctx->d_hex, at + 2 * nbytes + 64)) return rc;
+    uint8_t* d_raw = (uint8_t*)ctx->d_hex.p;
+    CU_TRY(ctx, cudaMemcpyAsync(d_raw, raw, nbytes, cudaMemcpyHostToDevice, ctx->s_comp));
+    ctx->launches += launch_hex_rows(d_raw, nbytes, d_raw + at, ctx->s_comp);
+    CU_TRY(ctx, cudaGetLastError());
+    CU_TRY(ctx, cudaMemcpyAsync(out, d_raw + at, 2 * nbytes, cudaMemcpyDefault, ctx->s_comp));
+    CU_TRY(ctx, cudaStreamSynchronize(ctx->s_comp));
+    return 0;
+}
+
 extern "C" {
 
 void b200h_destroy(b200h_ctx* ctx) {

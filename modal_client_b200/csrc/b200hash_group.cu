@@ -277,9 +277,10 @@ int scatter_device(Member& m, const Columns& c, Share& s, const size_t* col_at, 
     return 0;
 }
 
-// What one worker does with its member's share: hash it into share-sized outputs, scatter the rows.
+// What one worker does with its member's share: hash it into share-sized outputs, scatter the rows.  device_rows: the
+// share's off[] are absolute addresses of parts resident on the member's device (b200h_group_hash_device_parts).
 void run_share(b200h_group* g, int j, const uint8_t* base, const char* const* paths, uint32_t flags, const Columns& c,
-               Share& s) {
+               Share& s, bool device_rows = false) {
     const auto t0 = Clock::now();
     Member& m = *g->members[j];
     const uint64_t rows = s.idx.size();
@@ -303,8 +304,12 @@ void run_share(b200h_group* g, int j, const uint8_t* base, const char* const* pa
         for (int k = 0; k < 3; ++k)
             if (c.out[k] && c.on_device[k]) to[k] = m.share.p + col_at[k];
     }
-    s.rc = b200h::hash_share(m.ctx, base, s.off.data(), s.len.data(), rows, flags, to[0], to[1], (uint64_t*)to[2], paths,
-                             paths ? s.file_of.data() : nullptr, &s.staged);
+    if (device_rows)
+        s.rc = b200h::hash_device_rows(m.ctx, s.off.data(), s.len.data(), rows, flags, to[0], to[1], (uint64_t*)to[2],
+                                       nullptr, 0, nullptr);
+    else
+        s.rc = b200h::hash_share(m.ctx, base, s.off.data(), s.len.data(), rows, flags, to[0], to[1], (uint64_t*)to[2],
+                                 paths, paths ? s.file_of.data() : nullptr, &s.staged);
     if (s.rc) {
         s.err = b200h_last_error(m.ctx);
     } else {
@@ -332,10 +337,13 @@ void record_split(b200h_group* g, const std::vector<Share>& shares) {
     }
 }
 
-// Deal messages (off, len, file_of) over the members, run every share on its member's worker, wait for all of them.
+// Deal messages (off, len, file_of) over the members (owner[i] = member of message i), run every non-empty share on
+// its member's worker, wait for all of them.
 int run_split(b200h_group* g, const uint8_t* base, const char* const* paths, const uint64_t* off, const uint64_t* len,
-              const uint64_t* file_of, uint64_t n, uint32_t flags, const Columns& c, int k, const uint32_t* owner) {
-    std::vector<Share> shares(k);
+              const uint64_t* file_of, uint64_t n, uint32_t flags, const Columns& c, const uint32_t* owner,
+              bool device_rows = false) {
+    const int nm = (int)g->members.size();
+    std::vector<Share> shares(nm);
     for (uint64_t i = 0; i < n; ++i) {
         Share& s = shares[owner[i]];
         s.idx.push_back(i);
@@ -346,21 +354,23 @@ int run_split(b200h_group* g, const uint8_t* base, const char* const* paths, con
     }
     std::mutex dm;
     std::condition_variable dcv;
-    int left = k;
-    for (int j = 0; j < k; ++j)
-        g->members[j]->worker->post([&, j] {
-            run_share(g, j, base, paths, flags, c, shares[j]);
-            std::lock_guard<std::mutex> lk(dm);  // notify under the lock: the waiter's cv lives on its stack
-            --left;
-            dcv.notify_one();
-        });
+    int left = 0;
+    for (int j = 0; j < nm; ++j) left += !shares[j].idx.empty();
+    for (int j = 0; j < nm; ++j)
+        if (!shares[j].idx.empty())
+            g->members[j]->worker->post([&, j] {
+                run_share(g, j, base, paths, flags, c, shares[j], device_rows);
+                std::lock_guard<std::mutex> lk(dm);  // notify under the lock: the waiter's cv lives on its stack
+                --left;
+                dcv.notify_one();
+            });
     {
         std::unique_lock<std::mutex> lk(dm);
         dcv.wait(lk, [&] { return left == 0; });
     }
     std::lock_guard<std::mutex> lk(g->mu);
     record_split(g, shares);
-    for (int j = 0; j < k; ++j)
+    for (int j = 0; j < nm; ++j)
         if (shares[j].rc) {
             g->err = member_prefix(g, j) + shares[j].err;
             return shares[j].rc;
@@ -368,22 +378,37 @@ int run_split(b200h_group* g, const uint8_t* base, const char* const* paths, con
     return 0;
 }
 
-// k <= 1: the home member's own entry point, exactly.
+// k <= 1: the home member's own entry point, exactly (or member j's, when the one member a batch uses is not home).
 template <typename F>
-int run_home(b200h_group* g, uint64_t n, const uint64_t* len, F call) {
-    b200h_ctx* home = g->members[0]->ctx;
+int run_home(b200h_group* g, uint64_t n, const uint64_t* len, F call, int j = 0) {
+    b200h_ctx* home = g->members[j]->ctx;
     const auto t0 = Clock::now();
     const uint64_t staged0 = b200h::staged_bytes(home);
     const int rc = call(home);
-    std::vector<Share> one(1);
-    one[0].idx.resize(n);
-    for (uint64_t i = 0; i < n; ++i) one[0].bytes += len[i];
-    one[0].staged = b200h::staged_bytes(home) - staged0;
-    one[0].ms = ms_since(t0);
+    std::vector<Share> one(j + 1);
+    one[j].idx.resize(n);
+    for (uint64_t i = 0; i < n; ++i) one[j].bytes += len[i];
+    one[j].staged = b200h::staged_bytes(home) - staged0;
+    one[j].ms = ms_since(t0);
     std::lock_guard<std::mutex> lk(g->mu);
     record_split(g, one);
-    if (rc) g->err = member_prefix(g, 0) + b200h_last_error(home);
+    if (rc) g->err = member_prefix(g, j) + b200h_last_error(home);
     return rc;
+}
+
+// The raw columns of a device-parts batch (hashed into host memory because ETags were asked for) into the caller's
+// outputs: copied as they are, or formatted as hex on the home member's device.
+int deliver_raw(b200h_group* g, const uint8_t* raw, uint64_t nbytes, uint8_t* out, bool hex) {
+    if (!out || !nbytes) return 0;
+    if (hex) {
+        b200h_ctx* home = g->members[0]->ctx;
+        if (int rc = b200h::hex_rows_from_host(home, raw, nbytes, out))
+            return group_fail(g, rc, member_prefix(g, 0) + b200h_last_error(home));
+        return 0;
+    }
+    const cudaError_t e = cudaMemcpy(out, raw, nbytes, cudaMemcpyDefault);
+    if (e != cudaSuccess) return group_fail(g, B200H_E_CUDA, cuda_msg("cudaMemcpy (group outputs)", e));
+    return 0;
 }
 
 }  // namespace
@@ -478,7 +503,7 @@ int b200h_group_hash_batch_host(b200h_group* g, const uint8_t* base, const uint6
     c.width[0] = 32 * wide;
     c.width[1] = 16 * wide;
     if (int rc = classify_outputs(g, c)) return rc;
-    return run_split(g, base, nullptr, offsets, lengths, nullptr, n, flags, c, k, owner.data());
+    return run_split(g, base, nullptr, offsets, lengths, nullptr, n, flags, c, owner.data());
 }
 
 int b200h_group_hash_files(b200h_group* g, const char* const* paths, uint64_t n, const uint64_t* sizes,
@@ -504,7 +529,101 @@ int b200h_group_hash_files(b200h_group* g, const char* const* paths, uint64_t n,
     c.width[0] = 32 * wide;
     c.width[1] = 16 * wide;
     if (int rc = classify_outputs(g, c)) return rc;
-    return run_split(g, nullptr, paths, off.data(), len.data(), file_of.data(), rows, flags, c, k, owner.data());
+    return run_split(g, nullptr, paths, off.data(), len.data(), file_of.data(), rows, flags, c, owner.data());
+}
+
+int b200h_group_hash_device_parts(b200h_group* g, const void* const* d_bufs, const uint64_t* sizes, uint64_t n,
+                                  uint64_t part_len, uint32_t flags, uint8_t* sha256_out, uint8_t* md5_out,
+                                  uint64_t* trimmed_len_out, uint8_t* etag_md5_out) {
+    if (!g) return B200H_E_INVALID;
+    if (n && (!d_bufs || !sizes)) return group_fail(g, B200H_E_INVALID, "d_bufs/sizes must not be NULL");
+    if (!(flags & (B200H_SHA256 | B200H_MD5))) return group_fail(g, B200H_E_INVALID, "flags select neither SHA256 nor MD5");
+    if (etag_md5_out && !(flags & B200H_MD5)) return group_fail(g, B200H_E_INVALID, "etag requires B200H_MD5");
+    const int nm = (int)g->members.size();
+    // where every buffer lives; a buffer may only be hashed by the members on its device
+    std::vector<int> buf_dev(n);
+    for (uint64_t i = 0; i < n; ++i) {
+        std::string what;
+        const int d = b200h::buffer_device(d_bufs[i], sizes[i], &what);
+        if (d == -1) return group_fail(g, B200H_E_INVALID, "buffer " + std::to_string(i) + " is " + what);
+        bool covered = d < 0;
+        for (int j = 0; j < nm && !covered; ++j) covered = g->members[j]->device == d;
+        if (!covered)
+            return group_fail(g, B200H_E_INVALID, "buffer " + std::to_string(i) + " is on cuda:" + std::to_string(d) +
+                                                      ", which is not in the group");
+        buf_dev[i] = d >= 0 ? d : g->members[0]->device;  // an empty buffer reads nothing: the home device takes it
+    }
+    std::vector<uint64_t> addr, len, row_of;
+    b200h::device_part_rows(d_bufs, sizes, n, part_len, addr, len, row_of);
+    const uint64_t rows = addr.size();
+    // the parts resident on device d are dealt over the members on d by the rule of every other group batch
+    std::vector<uint32_t> owner(rows);
+    std::vector<int> used;
+    std::vector<int> devs(buf_dev.begin(), buf_dev.end());
+    std::sort(devs.begin(), devs.end());
+    devs.erase(std::unique(devs.begin(), devs.end()), devs.end());
+    for (int d : devs) {
+        std::vector<uint64_t> idx, dlen;
+        for (uint64_t b = 0; b < n; ++b)
+            if (buf_dev[b] == d)
+                for (uint64_t r = row_of[b]; r < row_of[b + 1]; ++r) {
+                    idx.push_back(r);
+                    dlen.push_back(len[r]);
+                }
+        if (idx.empty()) continue;
+        std::vector<int> on_d;
+        for (int j = 0; j < nm; ++j)
+            if (g->members[j]->device == d) on_d.push_back(j);
+        std::vector<uint32_t> local(idx.size());
+        const int k = split_owner(dlen.data(), idx.size(), (int)on_d.size(), g->min_share, local.data());
+        for (size_t p = 0; p < idx.size(); ++p) owner[idx[p]] = (uint32_t)on_d[local[p]];
+        for (int q = 0; q < k; ++q) used.push_back(on_d[q]);
+    }
+    if (used.size() <= 1)
+        return run_home(
+            g, rows, len.data(),
+            [&](b200h_ctx* m) {
+                return b200h_hash_device_parts(m, d_bufs, sizes, n, part_len, flags, sha256_out, md5_out, trimmed_len_out,
+                                               etag_md5_out);
+            },
+            used.empty() ? 0 : used[0]);
+    const uint32_t wide = (flags & B200H_HEX_OUT) ? 2 : 1;
+    Columns c;
+    if (!etag_md5_out) {
+        c.out[0] = (flags & B200H_SHA256) ? sha256_out : nullptr;
+        c.out[1] = (flags & B200H_MD5) ? md5_out : nullptr;
+        c.out[2] = (uint8_t*)trimmed_len_out;
+        c.width[0] = 32 * wide;
+        c.width[1] = 16 * wide;
+        if (int rc = classify_outputs(g, c)) return rc;
+        return run_split(g, nullptr, nullptr, addr.data(), len.data(), nullptr, rows, flags, c, owner.data(), true);
+    }
+    // ETags need every raw MD5 row in one place: the shares land in host tables, the ETags are one batch over
+    // segments of the MD5 table on the home member, then the columns go where the caller wants them.
+    std::vector<uint8_t> tsha((flags & B200H_SHA256) ? rows * 32 : 0), tmd5(rows * 16 + 16);
+    std::vector<uint64_t> ttrim(rows);
+    c.out[0] = tsha.empty() ? nullptr : tsha.data();
+    c.out[1] = tmd5.data();
+    c.out[2] = (uint8_t*)ttrim.data();
+    c.width[0] = 32;
+    c.width[1] = 16;
+    if (int rc = run_split(g, nullptr, nullptr, addr.data(), len.data(), nullptr, rows, flags & ~B200H_HEX_OUT, c,
+                           owner.data(), true))
+        return rc;
+    std::vector<uint64_t> eoff(n), elen(n);
+    for (uint64_t b = 0; b < n; ++b) {
+        eoff[b] = 16 * row_of[b];
+        elen[b] = 16 * (row_of[b + 1] - row_of[b]);
+    }
+    b200h_ctx* home = g->members[0]->ctx;
+    uint64_t staged = 0;
+    if (int rc = b200h::hash_share(home, tmd5.data(), eoff.data(), elen.data(), n, B200H_MD5, nullptr, etag_md5_out,
+                                   nullptr, nullptr, nullptr, &staged))
+        return group_fail(g, rc, member_prefix(g, 0) + b200h_last_error(home));
+    const bool hex = (flags & B200H_HEX_OUT) != 0;
+    if (int rc = deliver_raw(g, tsha.data(), tsha.size(), sha256_out, hex)) return rc;
+    if (int rc = deliver_raw(g, tmd5.data(), rows * 16, md5_out, hex)) return rc;
+    return deliver_raw(g, (const uint8_t*)ttrim.data(), rows * 8, (uint8_t*)trimmed_len_out, false);
 }
 
 int b200h_group_last_split(b200h_group* g, uint64_t* messages_out, uint64_t* bytes_out, uint64_t* staged_bytes_out,

@@ -1,8 +1,10 @@
-// b200hash_internal.h -- what a device group (b200hash_group.cu) needs from its member contexts beyond the C ABI.
+// b200hash_internal.h -- what a device group (b200hash_group.cu) and the device-buffer entry points
+// (b200hash_device_parts.cu) need from a context beyond the C ABI.
 #pragma once
 #include <stddef.h>
 #include <stdint.h>
 
+#include <string>
 #include <vector>
 
 #include "../../include/b200hash.h"
@@ -29,5 +31,32 @@ uint64_t staged_bytes(b200h_ctx* ctx);
 // The message list of b200h_hash_files: one per file (part_len == 0) or one per part_len-sized part, file-major.
 void file_messages(const uint64_t* sizes, uint64_t n, uint64_t part_len, std::vector<uint64_t>& off,
                    std::vector<uint64_t>& len, std::vector<uint64_t>& file_of);
+
+// ---- device-resident buffers (b200hash_device_parts.cu) ----
+
+// The CUDA device ctx is bound to, and ctx's last_error set to msg (returns code).
+int ctx_device(b200h_ctx* ctx);
+int ctx_fail(b200h_ctx* ctx, int code, const std::string& msg);
+
+// Where [d_bufs[i], +sizes[i]) lives: the device index, or -1 with *what set ("host memory", ...) when it is not
+// device memory.  A zero-size buffer is nowhere (returns -2) and may be any pointer.
+int buffer_device(const void* p, uint64_t size, std::string* what);
+
+// The row table of b200h_hash_device_parts: absolute device addresses and lengths of every part, file-major, and the
+// first row of every buffer (row_of[n] = rows).
+void device_part_rows(const void* const* d_bufs, const uint64_t* sizes, uint64_t n, uint64_t part_len,
+                      std::vector<uint64_t>& addr, std::vector<uint64_t>& len, std::vector<uint64_t>& row_of);
+
+// Hash `rows` device-resident messages (absolute addresses, on ctx's device; a zero-length row may hold any address)
+// on ctx: the row table goes to the device in one copy, then trim -> plan -> lane/chain on the context's stream with
+// the lengths known on the host.  etag_out (n*16, may be NULL) = MD5 over the raw MD5 rows [row_of[i], row_of[i+1])
+// of buffer i, one more lane_hash launch.  Outputs may be host or device memory; returns when they are written.
+int hash_device_rows(b200h_ctx* ctx, const uint64_t* addr, const uint64_t* len, uint64_t rows, uint32_t flags,
+                     uint8_t* sha_out, uint8_t* md5_out, uint64_t* trim_out, const uint64_t* row_of, uint64_t n,
+                     uint8_t* etag_out);
+
+// rows x width raw digest bytes in host memory -> lowercase hex rows (2 x width) at out (host or device), formatted
+// on ctx's device.
+int hex_rows_from_host(b200h_ctx* ctx, const uint8_t* raw, uint64_t nbytes, uint8_t* out);
 
 }  // namespace b200h

@@ -7,7 +7,8 @@ zero-trimmed 8 MiB block, ``VolumePutFiles2`` missing-block loop, :1345-1574).  
 hashes file by file (ThreadPoolExecutor) or block by block (``to_thread`` under a semaphore); here every path
 queued in the batch is handed to ``blob_utils.get_file_upload_specs`` / ``file_upload_specs2`` -- ONE GPU
 batch for the whole tree -- before the first RPC goes out.  File objects (``BytesIO`` / open files) keep the
-per-object spec builders.
+per-object spec builders.  CUDA tensors (``put_tensor``) are hashed in HBM by ``blob_utils.tensor_upload_specs`` /
+``tensor_upload_specs2`` -- one device call per batch -- and read back only for the bytes that are sent.
 """
 from __future__ import annotations
 
@@ -44,6 +45,7 @@ class _BatchBase:
         self._force = force
         self._paths: list[tuple[Path | str, str, int | None]] = []  # (local path, remote posix path, mode)
         self._fileobjs: list[tuple[BinaryIO, PurePosixPath, int]] = []
+        self._tensors: list[tuple[blob_utils.DeviceBufferReader, str, int]] = []
 
     async def __aenter__(self):
         return self
@@ -58,6 +60,40 @@ class _BatchBase:
         else:
             self._fileobjs.append((local_file, PurePosixPath(remote), mode or 0o644))
 
+    def put_tensor(self, tensor, remote_path: PurePosixPath | str, mode: int | None = None):
+        """Queue the raw bytes of a contiguous CUDA tensor (or a ``function_utils.DevicePayload``) as one file at
+        ``remote_path`` (mode 0o644 unless given): ``numel * element_size`` bytes from ``data_ptr()``, any dtype, no
+        header (``torch.save`` / safetensors framing is the caller's business).
+
+        The bytes are hashed where they are, on the GPU that holds them (each GPU of a device group hashes its own
+        tensors), in one call for all tensors of the batch; only bytes that must be sent are copied to the host, through
+        a small pinned buffer.  volumefs2 sends the zero-trimmed 8 MiB blocks the server reports missing, so re-saving
+        mostly unchanged weights moves little.  volumefs1 needs a whole-tensor SHA-256 (+ MD5 up to 1 GiB): each is one
+        serial chain on the device, about 71 MB/s -- roughly 15 s per GiB -- and the whole content is uploaded when
+        the server lacks it.
+
+        Work already queued on the tensor's current stream is part of what is uploaded.  The tensor must not be modified
+        (nor freed and reused) until the batch exits, like a queued file object.  Raises ``ValueError`` now for a
+        non-CUDA or non-contiguous tensor, a tensor on a device the current context or device group does not cover, or
+        a ``remote_path`` that ends in ``/``."""
+        from .function_utils import DevicePayload
+
+        remote = PurePosixPath(remote_path).as_posix()
+        if remote.endswith("/"):
+            raise ValueError(f"remote_path ({remote}) must refer to a file - cannot end with /")
+        if isinstance(tensor, DevicePayload):
+            tensor = tensor.tensor
+        if not getattr(tensor, "is_cuda", False):
+            raise ValueError(f"put_tensor needs a CUDA tensor, got {getattr(tensor, 'device', type(tensor).__name__)}; "
+                             "queue host data with put_file")
+        if not tensor.is_contiguous():
+            raise ValueError("put_tensor needs a contiguous tensor: call .contiguous() first")
+        covered = _context_devices(blob_utils.get_context())
+        if covered is not None and tensor.device.index not in covered:
+            raise ValueError(f"the tensor is on cuda:{tensor.device.index}, which the current context / device group "
+                             f"does not cover (devices {sorted(set(covered))})")
+        self._tensors.append((blob_utils.DeviceBufferReader(tensor), remote, mode or 0o644))
+
     def put_directory(self, local_path: Path | str, remote_path: PurePosixPath | str, recursive: bool = True):
         """Queue every regular file below ``local_path`` (directories and special files are skipped).
 
@@ -71,6 +107,15 @@ class _BatchBase:
         append = self._paths.append
         for abs_path, rel_posix in _walk_files(os.fspath(local_path), recursive):
             append((abs_path, f"{remote_root}/{rel_posix}", None))
+
+
+def _context_devices(ctx) -> list[int] | None:
+    """CUDA devices a context (one device) or a device group (its members' devices) hashes on; None when unknown."""
+    devices = getattr(ctx, "devices", None)
+    if devices is None:
+        device = getattr(ctx, "device", None)
+        devices = None if device is None or device < 0 else [device]
+    return devices
 
 
 def _walk_files(root: str, recursive: bool):
@@ -109,6 +154,7 @@ class VolumeUploadContextManager(_BatchBase):
         specs: list[FileUploadSpec] = await asyncio.to_thread(blob_utils.get_file_upload_specs, self._paths)
         for fp, remote, mode in self._fileobjs:
             specs.append(await asyncio.to_thread(blob_utils.get_file_upload_spec_from_fileobj, fp, remote, mode))
+        specs.extend(await asyncio.to_thread(blob_utils.tensor_upload_specs, self._tensors))
         logger.debug(f"Computed checksums for {len(specs)} files on the GPU")
         # In-batch dedupe on the digest table, computed on the GPU (b200h_dedupe_host; what Mount does with a set,
         # py/modal/mount.py:498,518-534): each distinct content is checked / uploaded once, however many paths carry
@@ -175,6 +221,7 @@ class VolumeUploadContextManager2(_BatchBase):
         one_at_a_time = asyncio.Semaphore(1)
         for fp, remote, mode in self._fileobjs:
             specs.append(await FileUploadSpec2.from_fileobj(fp, remote, one_at_a_time, mode))
+        specs.extend(await asyncio.to_thread(blob_utils.tensor_upload_specs2, self._tensors))
         await self._put_file_specs(specs)
 
     async def _put_file_specs(self, file_specs: list[FileUploadSpec2]):
@@ -267,6 +314,8 @@ class _AbstractVolumeUploadContextManager:
     def put_file(self, local_file, remote_path, mode=None): ...
 
     def put_directory(self, local_path, remote_path, recursive=True): ...
+
+    def put_tensor(self, tensor, remote_path, mode=None): ...
 
     @staticmethod
     def resolve(version, object_id: str, client, progress_cb: Callable[..., Any] | None = None, force: bool = False):
