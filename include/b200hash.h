@@ -133,6 +133,35 @@ int b200h_hash_device_parts(b200h_ctx* ctx, const void* const* d_bufs, const uin
                             uint64_t part_len, uint32_t flags, uint8_t* sha256_out, uint8_t* md5_out,
                             uint64_t* trimmed_len_out, uint8_t* etag_md5_out);
 
+/* File i = the concatenation of segments [seg_of[i], seg_of[i+1]) (seg_of has n_files+1 entries, non-decreasing); every
+ * non-empty segment is device memory on ctx's device, any alignment, any length (0 allowed).  Rows, flags and outputs
+ * exactly as b200h_hash_device_parts over the concatenated bytes of each file: the rows are bit for bit those of
+ * b200h_hash_device_parts on one buffer per file.  A safetensors file is one such file: its header, then its tensors.
+ * A part that lies in one segment is hashed where it is.  A part that straddles segments (zero-size segments are not
+ * boundaries) is gathered into a scratch buffer on ctx's device first, by one gather_pieces_kernel launch, and every
+ * part of the call goes to the hash kernels in ONE batch -- a batch of 8 MiB blocks costs about one block's chain,
+ * whatever the count.  Scratch holds every gathered part at once: at most min(file bytes, boundaries x part_len), and
+ * with part_len == 0 a file of several non-empty segments is gathered whole.  The scratch is capped by
+ * B200H_GATHER_BYTES (bytes, default 4 GiB): past the cap the gathered parts are hashed in successive windows (each
+ * one gather + one batch), correct but slower; a single part larger than the cap is a window of its own.  The scratch
+ * is allocated per call and freed before it returns; failing to allocate it is B200H_E_NOMEM, last_error giving the
+ * size.  A segment that is not device memory on ctx's device is B200H_E_INVALID, last_error naming the file, the
+ * segment index and where it lives. */
+int b200h_hash_device_segments(b200h_ctx* ctx, const void* const* d_segs, const uint64_t* seg_sizes,
+                               const uint64_t* seg_of, uint64_t n_files, uint64_t part_len, uint32_t flags,
+                               uint8_t* sha256_out, uint8_t* md5_out, uint64_t* trimmed_len_out,
+                               uint8_t* etag_md5_out);
+/* The row table of b200h_hash_device_segments alone, from the sizes: no context, no GPU.  window_bytes 0 = the
+ * B200H_GATHER_BYTES cap.  *n_rows_out = rows, *n_windows_out = windows (>= 1: contiguous row ranges, every window but
+ * the first starting at a gathered row).  Per row r (arrays of n_rows, each may be NULL): gathered_out[r] = 0 for a
+ * row hashed in place, with a_out[r] = its segment index and b_out[r] = its offset in that segment (an empty file's
+ * one row: segment seg_of[i], offset 0); gathered_out[r] = 1 for a gathered row, with a_out[r] = its window and
+ * b_out[r] = its number of pieces.  window_bytes_out[w] (n_windows entries, may be NULL) = scratch bytes of window w:
+ * its gathered rows, each rounded up to 16 bytes.  Call with NULL arrays first to learn the counts.  Diagnostic. */
+int b200h_segments_preview(const uint64_t* seg_sizes, const uint64_t* seg_of, uint64_t n_files, uint64_t part_len,
+                           uint64_t window_bytes, uint64_t* n_rows_out, uint64_t* n_windows_out, uint8_t* gathered_out,
+                           uint64_t* a_out, uint64_t* b_out, uint64_t* window_bytes_out);
+
 /* ---- files (native reader pool; no Python I/O, no mmap) ------------------------------------------ */
 
 /* Sizes (and permission bits, may be NULL) of n regular files, stat'ed by the library's I/O threads.
@@ -261,6 +290,15 @@ int b200h_group_hash_files(b200h_group* g, const char* const* paths, uint64_t n,
 int b200h_group_hash_device_parts(b200h_group* g, const void* const* d_bufs, const uint64_t* sizes, uint64_t n,
                                   uint64_t part_len, uint32_t flags, uint8_t* sha256_out, uint8_t* md5_out,
                                   uint64_t* trimmed_len_out, uint8_t* etag_md5_out);
+/* As b200h_hash_device_segments.  Every file's non-empty segments must be on one device ("file 2 has segments on
+ * cuda:0 and cuda:1" otherwise, B200H_E_INVALID; the group stays usable).  The rows of the files on device d are dealt
+ * over the members on d as in b200h_group_hash_device_parts; a member gathers the straddling rows of its own share into
+ * its own scratch (capped per member by B200H_GATHER_BYTES).  When one member takes the whole batch this IS
+ * b200h_hash_device_segments on that member. */
+int b200h_group_hash_device_segments(b200h_group* g, const void* const* d_segs, const uint64_t* seg_sizes,
+                                     const uint64_t* seg_of, uint64_t n_files, uint64_t part_len, uint32_t flags,
+                                     uint8_t* sha256_out, uint8_t* md5_out, uint64_t* trimmed_len_out,
+                                     uint8_t* etag_md5_out);
 /* What the last batch call did, per member (arrays of b200h_group_size entries, each may be NULL): messages, payload
  * bytes, bytes that went through the member's pinned staging ring (0 = DMAed straight from the caller's page-locked
  * memory) and wall milliseconds spent inside the member.  Members the batch did not use report zeros. */

@@ -36,6 +36,7 @@ ABI_SYMBOLS = (
     "b200h_group_create", "b200h_group_destroy", "b200h_group_last_error", "b200h_group_size", "b200h_group_member",
     "b200h_group_hash_batch_host", "b200h_group_hash_files", "b200h_group_last_split", "b200h_group_split_preview",
     "b200h_hash_device_parts", "b200h_group_hash_device_parts",
+    "b200h_hash_device_segments", "b200h_group_hash_device_segments", "b200h_segments_preview",
 )
 
 
@@ -45,7 +46,8 @@ class B200HashError(RuntimeError):
 
 def build_library(force: bool = False, verbose: bool = False) -> str:
     srcs = [os.path.join(CSRC, f) for f in ("b200hash_kernels.cu", "b200hash_dedupe.cu", "b200hash_api.cu",
-                                            "b200hash_group.cu", "b200hash_device_parts.cu", "b200hash_internal.h", "b200blob_host.cpp",
+                                            "b200hash_group.cu", "b200hash_device_parts.cu", "b200hash_device_segments.cu",
+                                            "b200hash_internal.h", "b200blob_host.cpp",
                                             "b200pack_copy.cpp", "b200hash_kernels.cuh", "b200pack_team.h")]
     srcs += [os.path.join(os.path.dirname(_PKG), "include", h) for h in ("b200hash.h", "b200blob.h")]
     stale = not os.path.exists(LIB_PATH) or any(os.path.getmtime(s) > os.path.getmtime(LIB_PATH) for s in srcs)
@@ -160,6 +162,12 @@ def load_library() -> ctypes.CDLL:
         L.b200h_hash_device_parts.restype = i32
         L.b200h_group_hash_device_parts.argtypes = [vp, vp, vp, u64, u64, u32, vp, vp, vp, vp]
         L.b200h_group_hash_device_parts.restype = i32
+        L.b200h_hash_device_segments.argtypes = [vp, vp, vp, vp, u64, u64, u32, vp, vp, vp, vp]
+        L.b200h_hash_device_segments.restype = i32
+        L.b200h_group_hash_device_segments.argtypes = [vp, vp, vp, vp, u64, u64, u32, vp, vp, vp, vp]
+        L.b200h_group_hash_device_segments.restype = i32
+        L.b200h_segments_preview.argtypes = [vp, vp, u64, u64, u64, ctypes.POINTER(u64), ctypes.POINTER(u64), vp, vp, vp, vp]
+        L.b200h_segments_preview.restype = i32
         _lib = L
         return L
 
@@ -198,6 +206,50 @@ def group_split_preview(lengths, nmembers: int, min_share_bytes: int = 0) -> tup
     if rc != 0:
         raise B200HashError(f"b200h_group_split_preview failed ({rc})")
     return owner[: ln.size], k.value
+
+
+def _segment_table(files) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+    """files: per file a sequence of (address, nbytes) segments -> (addresses, sizes, seg_of[n_files + 1])."""
+    counts = [len(f) for f in files]
+    seg_of = np.zeros(len(files) + 1, np.uint64)
+    np.cumsum(counts, out=seg_of[1:])
+    segs = [s for f in files for s in f]
+    addr = np.fromiter((int(a) for a, _ in segs), dtype=np.uint64, count=len(segs))
+    size = np.fromiter((int(n) for _, n in segs), dtype=np.uint64, count=len(segs))
+    return addr, size, seg_of
+
+
+def _segment_rows(sizes: np.ndarray, seg_of: np.ndarray, part_len: int) -> int:
+    csum = np.zeros(sizes.size + 1, np.uint64)
+    np.cumsum(sizes, out=csum[1:])
+    file_sizes = csum[seg_of[1:].astype(np.int64)] - csum[seg_of[:-1].astype(np.int64)]
+    return int(file_sizes.size) if part_len == 0 else int(((file_sizes + np.uint64(part_len - 1)) // np.uint64(part_len)).sum())
+
+
+def segments_preview(seg_sizes, seg_of, part_len: int, window_bytes: int = 0) -> dict:
+    """The row table ``b200h_hash_device_segments`` builds for files made of segments of these sizes (file i = segments
+    [seg_of[i], seg_of[i + 1])) -- the library's own code, no context, no GPU.  ``window_bytes`` 0 = the
+    B200H_GATHER_BYTES cap.  -> {"gathered": bool[rows], "a": uint64[rows], "b": uint64[rows],
+    "window_bytes": uint64[windows]}: an in-place row has a = segment, b = offset in it; a gathered row has a = window,
+    b = pieces."""
+    L = load_library()
+    sz = np.ascontiguousarray(seg_sizes, dtype=np.uint64)
+    so = np.ascontiguousarray(seg_of, dtype=np.uint64)
+    nf = max(int(so.size) - 1, 0)
+    rows, wins = ctypes.c_uint64(), ctypes.c_uint64()
+    args = (_np_ptr(sz) if sz.size else None, _np_ptr(so) if so.size else None, nf, part_len, window_bytes)
+    rc = L.b200h_segments_preview(*args, ctypes.byref(rows), ctypes.byref(wins), None, None, None, None)
+    if rc != 0:
+        raise B200HashError(f"b200h_segments_preview failed ({rc})")
+    g = np.zeros(max(rows.value, 1), np.uint8)
+    a, b = np.zeros(max(rows.value, 1), np.uint64), np.zeros(max(rows.value, 1), np.uint64)
+    wb = np.zeros(max(wins.value, 1), np.uint64)
+    rc = L.b200h_segments_preview(*args, ctypes.byref(rows), ctypes.byref(wins), _np_ptr(g), _np_ptr(a), _np_ptr(b),
+                                  _np_ptr(wb))
+    if rc != 0:
+        raise B200HashError(f"b200h_segments_preview failed ({rc})")
+    r, w = rows.value, wins.value
+    return {"gathered": g[:r].astype(bool), "a": a[:r], "b": b[:r], "window_bytes": wb[:w]}
 
 
 def pack_preview(base, offsets, lengths, threads: int = 16, slot_bytes: int = 256 << 20, dst: np.ndarray | None = None):
@@ -412,6 +464,32 @@ class Context:
     def _device_parts(self, *args):
         self._check(self._L.b200h_hash_device_parts(self._h, *args), "b200h_hash_device_parts")
 
+    # -- files made of device segments, e.g. a safetensors header plus its tensors (b200h_hash_device_segments)
+    def hash_device_segments(self, files, part_len: int, flags: int = SHA256 | MD5, want_etag: bool = False, *,
+                             out_sha: int = 0, out_md5: int = 0, out_trimmed: int = 0, out_etag: int = 0):
+        """files: per file, a sequence of ``(device address, nbytes)`` segments on this context's device; the file is
+        their concatenation.  Rows and results exactly as ``hash_device_parts`` with one buffer per file holding those
+        bytes: -> (sha[rows,32]|None, md5[rows,16]|None, trimmed[rows], etags[n,16]|None).  Parts that straddle
+        segments are gathered into scratch on the device first (B200H_GATHER_BYTES caps it)."""
+        addr, sz, seg_of = _segment_table(files)
+        n = len(files)
+        rows = _segment_rows(sz, seg_of, part_len)
+        wide = 2 if flags & HEX_OUT else 1
+        sha = np.empty((rows, 32 * wide), np.uint8) if (flags & SHA256 and not out_sha) else None
+        md5 = np.empty((rows, 16 * wide), np.uint8) if (flags & MD5 and not out_md5) else None
+        trimmed = None if out_trimmed else np.empty(rows, np.uint64)
+        etag = np.empty((n, 16), np.uint8) if (want_etag and not out_etag) else None
+        self._device_segments(_np_ptr(addr) if addr.size else None, _np_ptr(sz) if sz.size else None,
+                              _np_ptr(seg_of), n, part_len, flags,
+                              ctypes.c_void_p(out_sha) if out_sha else _np_ptr(sha),
+                              ctypes.c_void_p(out_md5) if out_md5 else _np_ptr(md5),
+                              ctypes.c_void_p(out_trimmed) if out_trimmed else _np_ptr(trimmed),
+                              ctypes.c_void_p(out_etag) if out_etag else _np_ptr(etag))
+        return sha, md5, trimmed, etag
+
+    def _device_segments(self, *args):
+        self._check(self._L.b200h_hash_device_segments(self._h, *args), "b200h_hash_device_segments")
+
     # -- files: stat + read + hash entirely inside the library (native reader threads, no mmap / Python I/O)
     @staticmethod
     def _c_paths(paths):
@@ -475,7 +553,8 @@ class Context:
 class DeviceGroup(Context):
     """One context per listed device, driven as one (include/b200hash.h, device groups).  ``hash_batch_host`` (and so
     ``hash_buffers``) and ``hash_files`` deal each batch over the members by bytes and hash the shares at the same time;
-    ``hash_device_parts`` deals the parts of device buffers over the members on each buffer's device;
+    ``hash_device_parts`` / ``hash_device_segments`` deal the parts of device buffers (files) over the members on each
+    buffer's (file's) device;
     every other method runs on the home member (``devices[0]``), whose handle this object carries as a Context.
     ``devices=None`` means every visible device; a device may repeat.  ``min_share_bytes`` 0 = the library default."""
 
@@ -510,6 +589,10 @@ class DeviceGroup(Context):
     def _device_parts(self, *args):
         # every buffer is hashed by the members on the device that holds it
         self._gcheck(self._L.b200h_group_hash_device_parts(self._g, *args), "b200h_group_hash_device_parts")
+
+    def _device_segments(self, *args):
+        # every file is hashed by the members on the device that holds its segments
+        self._gcheck(self._L.b200h_group_hash_device_segments(self._g, *args), "b200h_group_hash_device_segments")
 
     def close(self):
         if getattr(self, "_g", None):

@@ -148,5 +148,25 @@ def hash_blocks_tensors(tensors: Sequence, part_len: int, *, sha256: bool = True
     return DigestTable(s, m, t)
 
 
+def hash_blocks_segments(files: Sequence[Sequence], part_len: int, *, sha256: bool = True, md5: bool = False,
+                         trim_zeros: bool = False, ctx: Context | None = None, ready: Sequence | None = None) -> DigestTable:
+    """``hash_blocks_tensors`` for files made of several tensors: file i is the raw bytes of the contiguous CUDA tensors
+    ``files[i]`` back to back (a safetensors file is its header as a uint8 tensor, then its tensors).  The rows are
+    exactly those of ``hash_blocks_tensors`` over one tensor per file holding the concatenated bytes, without building
+    it: ``b200h_hash_device_segments`` gathers only the parts that straddle two tensors.  ``ready`` as for
+    ``hash_blocks_tensors`` (default: one event per tensor, recorded now)."""
+    ctx = ctx or get_context()
+    for f in files:
+        for t in f:
+            if not (getattr(t, "is_cuda", False) and t.is_contiguous()):
+                raise ValueError("hash_blocks_segments needs contiguous CUDA tensors")
+    for ev in (ready if ready is not None else [ready_event(t) for f in files for t in f]):
+        ev.synchronize()
+    flags = (SHA256 if sha256 else 0) | (MD5 if md5 else 0) | (TRIM_ZEROS if trim_zeros else 0)
+    s, m, t, _ = ctx.hash_device_segments([[(x.data_ptr(), x.numel() * x.element_size()) for x in f] for f in files],
+                                          part_len, flags)
+    return DigestTable(s, m, t)
+
+
 __all__ = ["DigestTable", "hash_table_host", "hash_table_buffers", "hash_table_tensors", "hash_blocks_tensors",
-           "ready_event", "Context", "default_context", "_lib"]
+           "hash_blocks_segments", "ready_event", "Context", "default_context", "_lib"]

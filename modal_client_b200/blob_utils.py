@@ -25,6 +25,7 @@ import dataclasses
 import functools
 import gc
 import io
+import json
 import mmap
 import os
 import platform
@@ -219,9 +220,9 @@ async def perform_multipart_upload(
     byte_budget: _ByteBudget | None = None,
 ) -> None:
     # 1. hash every part on the GPU before sending anything
-    on_device = isinstance(data_file, DeviceBufferReader)
-    start_pos = data_file.tell() if isinstance(data_file, (BytesIO, DeviceBufferReader)) else 0
-    if on_device:  # a tensor's bytes: the parts are hashed where they are, nothing is copied to the host for it
+    on_device = isinstance(data_file, (DeviceBufferReader, DeviceSegmentsReader))
+    start_pos = data_file.tell() if isinstance(data_file, (BytesIO, DeviceBufferReader, DeviceSegmentsReader)) else 0
+    if on_device:  # tensors' bytes: the parts are hashed where they are, nothing is copied to the host for it
         part_md5, expected_etag = await asyncio.to_thread(data_file.part_digests, start_pos, content_length, max_part_size)
     else:
         part_md5, expected_etag = await asyncio.to_thread(
@@ -1012,7 +1013,10 @@ class DeviceBufferReader(io.RawIOBase):
         super().close()
 
     def _copy(self, at: int, dst: np.ndarray) -> None:
-        src = self._flat[at : at + dst.size]
+        self._stage(self._flat[at : at + dst.size], dst)
+
+    def _stage(self, src, dst: np.ndarray) -> None:
+        """dst[:] = the uint8 tensor ``src``, through the pinned staging buffer when it is on the GPU."""
         if not src.is_cuda:
             dst[:] = src.numpy()
             return
@@ -1029,6 +1033,85 @@ class DeviceBufferReader(io.RawIOBase):
                 self._pin[:k].copy_(src[o : o + k], non_blocking=True)
                 self._stream.synchronize()
                 dst[o : o + k] = self._pin_np[:k]
+
+
+class DeviceSegmentsReader(DeviceBufferReader):
+    """Read-only, seekable binary file object over a file made of segments: ``header`` (host bytes) followed by the
+    raw bytes of contiguous ``tensors``, back to back -- a safetensors file whose tensors stay in HBM.  Reads, clones,
+    ``bytes_to_host`` and ``wait_ready`` behave as for ``DeviceBufferReader``; a read of the header range is served
+    from the host bytes (and counted like any other byte read).  The header also lives in a small CUDA tensor on the
+    tensors' device, so the hash calls see device segments only.  The ready event is recorded on the device's current
+    stream when the reader is made.  With CPU tensors every read is a plain copy (host-backed reader, for host-side
+    tests)."""
+
+    def __init__(self, header: bytes, tensors: Sequence, *, stage_bytes: int = 4 << 20,
+                 _root: "DeviceSegmentsReader | None" = None):
+        io.RawIOBase.__init__(self)
+        if _root is None:
+            torch = _torch()
+            self.header = bytes(header)
+            self.tensors = list(tensors)
+            self._flats = [t.reshape(-1).view(torch.uint8) for t in self.tensors]
+            dev = self.tensors[0].device if self.tensors else torch.device("cpu")
+            host_header = torch.frombuffer(bytearray(self.header), dtype=torch.uint8)
+            self._header_t = host_header.to(dev) if dev.type == "cuda" else host_header
+            sizes = [len(self.header)] + [int(f.numel()) for f in self._flats]
+            self._starts = np.concatenate([[0], np.cumsum(sizes)]).astype(np.int64)
+            self.nbytes = int(self._starts[-1])
+            self._counter = _ByteCounter()
+            self._ready = None
+            if dev.type == "cuda":
+                from .batch import ready_event
+
+                self._ready = ready_event(self._header_t)
+        else:
+            self.header, self.tensors, self._flats, self._header_t = _root.header, _root.tensors, _root._flats, _root._header_t
+            self._starts, self.nbytes, self._counter, self._ready = _root._starts, _root.nbytes, _root._counter, _root._ready
+        self._stage_bytes = stage_bytes
+        self._pos = 0
+        self._pin = self._pin_np = self._stream = None
+
+    @property
+    def data_ptr(self) -> int:
+        raise TypeError("a DeviceSegmentsReader has no single buffer: use segments()")
+
+    @property
+    def device(self):
+        return self._header_t.device
+
+    def segments(self, start: int = 0, length: int | None = None) -> list[tuple[int, int]]:
+        """(device address, nbytes) of the pieces of the header tensor and the tensors that make up bytes
+        [start, start + length) of the file: the segment list of ``hash_device_segments``."""
+        end = self.nbytes if length is None else start + length
+        out = []
+        for i, t in enumerate([self._header_t] + self._flats):
+            lo, hi = max(start, int(self._starts[i])), min(end, int(self._starts[i + 1]))
+            if hi > lo:
+                out.append((t.data_ptr() + lo - int(self._starts[i]), hi - lo))
+        return out
+
+    def clone(self) -> "DeviceSegmentsReader":
+        return DeviceSegmentsReader(b"", (), stage_bytes=self._stage_bytes, _root=self)
+
+    def part_digests(self, start: int, length: int, part_length: int) -> tuple[list[bytes], str]:
+        """``multipart_part_digests`` of bytes [start, start + length), hashed on the device where they are: the part
+        MD5s and the multipart ETag from one ``b200h_hash_device_segments(part_length, MD5)`` call."""
+        self.wait_ready()
+        _, md5, _, etag = get_context().hash_device_segments([self.segments(start, length)], part_length, _lib.MD5,
+                                                             want_etag=True)
+        return [md5[i].tobytes() for i in range(len(md5))], f"{etag[0].tobytes().hex()}-{len(md5)}"
+
+    def _copy(self, at: int, dst: np.ndarray) -> None:
+        end = at + dst.size
+        hl = len(self.header)
+        if at < hl:
+            k = min(end, hl) - at
+            dst[:k] = np.frombuffer(self.header, np.uint8, count=k, offset=at)
+        for i, f in enumerate(self._flats):
+            lo, hi = max(at, int(self._starts[i + 1])), min(end, int(self._starts[i + 2]))
+            if hi > lo:
+                base = int(self._starts[i + 1])
+                self._stage(f[lo - base : hi - base], dst[lo - at : hi - at])
 
 
 def _torch():
@@ -1091,6 +1174,103 @@ def tensor_upload_specs2(items: Sequence[tuple[DeviceBufferReader, PurePosixPath
             blocks.append(FileUploadBlock(start, start + trimmed_l[row], sha_raw[32 * row : 32 * row + 32]))
             row += 1
         out.append(FileUploadSpec2(source=r.clone, source_description=f"<tensor {tuple(r.tensor.shape)} {r.tensor.dtype}>",
+                                   path=PurePosixPath(remote).as_posix(), blocks=blocks, mode=mode & 0o7777,
+                                   size=r.nbytes))
+    return out
+
+
+# ------------------------------------------------------------------------- safetensors files straight from HBM
+
+# safetensors dtype names in data order (the library sorts tensors by this rank, then by name), as torch dtype names
+_SAFETENSORS_DTYPES = (
+    ("U64", "uint64"), ("I64", "int64"), ("F64", "float64"), ("C64", "complex64"), ("F32", "float32"),
+    ("U32", "uint32"), ("I32", "int32"), ("BF16", "bfloat16"), ("F16", "float16"), ("U16", "uint16"),
+    ("I16", "int16"), ("F8_E4M3", "float8_e4m3fn"), ("F8_E5M2", "float8_e5m2"), ("I8", "int8"), ("U8", "uint8"),
+    ("BOOL", "bool"),
+)
+
+
+def safetensors_layout(tensors, metadata: dict[str, str] | None = None) -> tuple[bytes, list[tuple[str, Any]]]:
+    """The safetensors framing of a state dict without the safetensors package: ``(header, [(name, tensor), ...])``
+    such that ``header`` followed by the raw bytes of the tensors in that order is byte for byte what
+    ``safetensors.torch.save(tensors, metadata)`` returns.  The header is the 8-byte little-endian length of the JSON,
+    then compact JSON (UTF-8, ``__metadata__`` first, then the tensors in data order: by dtype rank, then name), padded
+    with spaces to a multiple of 8.  A dtype safetensors cannot store is a ``ValueError`` naming the tensor."""
+    torch = _torch()
+    rank = {getattr(torch, tn): (i, st) for i, (st, tn) in enumerate(_SAFETENSORS_DTYPES) if hasattr(torch, tn)}
+    keyed = []
+    for name, t in tensors.items():
+        if t.dtype not in rank:
+            raise ValueError(f"tensor {name!r} has dtype {t.dtype}, which safetensors cannot store")
+        keyed.append((rank[t.dtype][0], name, t))
+    keyed.sort(key=lambda x: (x[0], x[1]))
+    head: dict[str, Any] = {}
+    if metadata is not None:
+        head["__metadata__"] = dict(metadata)
+    at = 0
+    for _, name, t in keyed:
+        n = t.numel() * t.element_size()
+        head[name] = {"dtype": rank[t.dtype][1], "shape": list(t.shape), "data_offsets": [at, at + n]}
+        at += n
+    js = json.dumps(head, ensure_ascii=False, separators=(",", ":")).encode("utf-8")
+    js += b" " * (-len(js) % 8)
+    return len(js).to_bytes(8, "little") + js, [(name, t) for _, name, t in keyed]
+
+
+def _segments_digests(readers: Sequence[DeviceSegmentsReader], part_len: int, flags: int):
+    """One ``hash_device_segments`` call over every reader's file, once the work queued before each was made is done."""
+    for r in readers:
+        r.wait_ready()
+    return get_context().hash_device_segments([r.segments() for r in readers], part_len, flags)
+
+
+def _safetensors_description(r: DeviceSegmentsReader) -> str:
+    return f"<safetensors: {len(r.tensors)} tensors, {r.nbytes} bytes>"
+
+
+def safetensors_upload_specs(items: Sequence[tuple[DeviceSegmentsReader, PurePosixPath | str, int]]) -> list[FileUploadSpec]:
+    """``FileUploadSpec`` (volumefs1) for files queued with ``put_safetensors``: whole-file SHA-256 (+ MD5 by
+    ``_size_class``) on the device.  A file of several segments is gathered whole into scratch first, then each digest
+    is ONE serial chain, about 71 MB/s (DESIGN §5.4): roughly 15 s per GiB."""
+    if not items:
+        return []
+    readers = [r for r, _, _ in items]
+    classes = [_size_class(r.nbytes) for r in readers]
+    sha_hex, md5_hex = [""] * len(items), [_MD5_PLACEHOLDER] * len(items)
+    for want_md5 in (True, False):
+        idx = [i for i, c in enumerate(classes) if c[1] == want_md5]
+        if not idx:
+            continue
+        sha, md5, _, _ = _segments_digests([readers[i] for i in idx], 0, _lib.SHA256 | (_lib.MD5 if want_md5 else 0))
+        for row, i in enumerate(idx):
+            sha_hex[i] = sha[row].tobytes().hex()
+            if want_md5:
+                md5_hex[i] = md5[row].tobytes().hex()
+    return [
+        FileUploadSpec(source=r.clone, source_description=_safetensors_description(r), source_is_path=False,
+                       mount_filename=PurePosixPath(remote).as_posix(), use_blob=classes[i][0], sha256_hex=sha_hex[i],
+                       md5_hex=md5_hex[i], mode=mode & 0o7777, size=r.nbytes)
+        for i, (r, remote, mode) in enumerate(items)
+    ]
+
+
+def safetensors_upload_specs2(items: Sequence[tuple[DeviceSegmentsReader, PurePosixPath | str, int]]) -> list[FileUploadSpec2]:
+    """``FileUploadSpec2`` (volumefs2) for files queued with ``put_safetensors``: every 8 MiB block of every file in ONE
+    ``hash_device_segments(BLOCK_SIZE, SHA256 | TRIM_ZEROS)`` call, the blocks exactly as ``file_upload_specs2`` builds
+    them from the same bytes.  Only the trimmed bytes of the blocks the server reports missing are copied to the host."""
+    if not items:
+        return []
+    readers = [r for r, _, _ in items]
+    bs = BLOCK_SIZE
+    sha, _, trimmed, _ = _segments_digests(readers, bs, _lib.SHA256 | _lib.TRIM_ZEROS)
+    trimmed_l, sha_raw = trimmed.tolist(), sha.tobytes()
+    out, row = [], 0
+    for r, remote, mode in items:
+        blocks = []
+        for start in range(0, r.nbytes, bs):
+            blocks.append(FileUploadBlock(start, start + trimmed_l[row], sha_raw[32 * row : 32 * row + 32]))
+            row += 1
+        out.append(FileUploadSpec2(source=r.clone, source_description=_safetensors_description(r),
                                    path=PurePosixPath(remote).as_posix(), blocks=blocks, mode=mode & 0o7777,
                                    size=r.nbytes))
     return out

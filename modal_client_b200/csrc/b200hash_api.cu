@@ -1046,7 +1046,7 @@ int b200h::ctx_fail(b200h_ctx* ctx, int code, const std::string& msg) {
 
 int b200h::hash_device_rows(b200h_ctx* ctx, const uint64_t* addr, const uint64_t* len, uint64_t rows, uint32_t flags,
                             uint8_t* sha_out, uint8_t* md5_out, uint64_t* trim_out, const uint64_t* row_of, uint64_t n,
-                            uint8_t* etag_out) {
+                            uint8_t* etag_out, const GatherRows* gather) {
     std::lock_guard<std::mutex> lk(ctx->mu);
     flags &= kPublicFlags;
     if (!(flags & (B200H_SHA256 | B200H_MD5))) return fail(ctx, B200H_E_INVALID, "flags select neither SHA256 nor MD5");
@@ -1054,20 +1054,67 @@ int b200h::hash_device_rows(b200h_ctx* ctx, const uint64_t* addr, const uint64_t
     const uint64_t ne = etag_out ? n : 0;
     if (rows == 0 && ne == 0) return 0;
     CU_TRY(ctx, cudaSetDevice(ctx->device));
-    // One pinned table -- addresses | lengths | ETag segment offsets | ETag segment lengths -- and one copy of it.
+    // Gathered rows: windows of rows (one, unless the gathered bytes pass the cap), a scratch buffer as large as the
+    // largest window, and the work items of gather_pieces_kernel (pieces split at gather_item_bytes), window-major.
+    std::vector<uint64_t> win{0, rows}, dst, win_bytes{0}, win_items{0, 0};
+    uint64_t items = 0, scratch_bytes = 0;
+    if (gather) {
+        gather_windows(len, gather->piece_of, rows, gather->window_bytes, win, dst, win_bytes);
+        win_items.assign(1, 0);
+        const uint64_t step = gather_item_bytes();
+        for (size_t w = 0; w + 1 < win.size(); ++w) {
+            for (uint64_t r = win[w]; r < win[w + 1]; ++r)
+                for (uint64_t p = gather->piece_of[r]; p < gather->piece_of[r + 1]; ++p) items += (gather->plen[p] + step - 1) / step;
+            win_items.push_back(items);
+            scratch_bytes = std::max(scratch_bytes, win_bytes[w]);
+        }
+    }
+    struct Scratch {
+        void* p = nullptr;
+        ~Scratch() {
+            if (p) cudaFree(p);
+        }
+    } scratch;
+    if (scratch_bytes) {
+        const cudaError_t e = cudaMalloc(&scratch.p, scratch_bytes);
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            scratch.p = nullptr;
+            return fail(ctx, e == cudaErrorMemoryAllocation ? B200H_E_NOMEM : B200H_E_CUDA,
+                        "cannot allocate " + std::to_string(scratch_bytes) + " bytes of gather scratch on cuda:" +
+                            std::to_string(ctx->device) + " (" + cudaGetErrorString(e) + ")");
+        }
+    }
+    // One pinned table -- addresses | lengths | ETag segment offsets | ETag segment lengths | gather sources |
+    // gather destinations | gather lengths -- and one copy of it.
     // A zero-length row reads nothing; it is pointed at library scratch so that no kernel ever sees a stray address.
-    if (int rc = ensure_meta(ctx, 2 * rows + 2 * ne)) return rc;
+    if (int rc = ensure_meta(ctx, 2 * rows + 2 * ne + 3 * items)) return rc;
     if (int rc = ensure_dev(ctx, ctx->d_small, 256)) return rc;
     uint64_t* h = ctx->h_meta;
     for (uint64_t i = 0; i < rows; ++i) {
-        h[i] = len[i] ? addr[i] : (uint64_t)(uintptr_t)ctx->d_small.p;
+        const bool gathered = gather && gather->piece_of[i + 1] > gather->piece_of[i];
+        h[i] = !len[i] ? (uint64_t)(uintptr_t)ctx->d_small.p : gathered ? (uint64_t)(uintptr_t)scratch.p + dst[i] : addr[i];
         h[rows + i] = len[i];
     }
     for (uint64_t b = 0; b < ne; ++b) {
         h[2 * rows + b] = 16 * row_of[b];
         h[2 * rows + ne + b] = 16 * (row_of[b + 1] - row_of[b]);
     }
-    const size_t table_bytes = (2 * rows + 2 * ne) * sizeof(uint64_t);
+    uint64_t* h_items = h + 2 * rows + 2 * ne;
+    if (items) {
+        const uint64_t step = gather_item_bytes();
+        uint64_t t = 0;
+        for (uint64_t r = 0; r < rows; ++r) {
+            uint64_t at = h[r];  // the row's place in scratch; its pieces follow one another there
+            for (uint64_t p = gather->piece_of[r]; p < gather->piece_of[r + 1]; at += gather->plen[p++])
+                for (uint64_t o = 0; o < gather->plen[p]; o += step, ++t) {
+                    h_items[t] = gather->psrc[p] + o;
+                    h_items[items + t] = at + o;
+                    h_items[2 * items + t] = std::min(step, gather->plen[p] - o);
+                }
+        }
+    }
+    const size_t table_bytes = (2 * rows + 2 * ne + 3 * items) * sizeof(uint64_t);
     if (int rc = ensure_dev(ctx, ctx->d_off, table_bytes)) return rc;
     if (int rc = ensure_dev(ctx, ctx->d_trim, rows * sizeof(uint64_t) + 8)) return rc;
     if (flags & B200H_SHA256)
@@ -1085,10 +1132,19 @@ int b200h::hash_device_rows(b200h_ctx* ctx, const uint64_t* addr, const uint64_t
     uint8_t* d_etag = hex_sha + rows * 96;
     CU_TRY(ctx, cudaMemcpyAsync(d_tab, h, table_bytes, cudaMemcpyHostToDevice, ctx->s_comp));
     // the lengths are known here: outliers are routed without a read-back (B200H_TRIM_ZEROS still needs its one)
-    if (rows)
-        if (int rc = enqueue_device_batch(ctx, nullptr, d_tab, d_tab + rows, rows, flags, d_sha, d_md5, d_trim, nullptr,
-                                          ctx->s_comp, len))
-            return rc;
+    const uint64_t* d_items = d_tab + 2 * rows + 2 * ne;
+    for (size_t w = 0; w + 1 < win.size(); ++w) {
+        const uint64_t r0 = win[w], nr = win[w + 1] - win[w], i0 = win_items[w], ni = win_items[w + 1] - win_items[w];
+        if (ni) {
+            ctx->launches += launch_gather(d_items + i0, d_items + items + i0, d_items + 2 * items + i0, ni, ctx->s_comp);
+            CU_TRY(ctx, cudaGetLastError());
+        }
+        if (nr)
+            if (int rc = enqueue_device_batch(ctx, nullptr, d_tab + r0, d_tab + rows + r0, nr, flags,
+                                              d_sha ? d_sha + 32 * r0 : nullptr, d_md5 ? d_md5 + 16 * r0 : nullptr,
+                                              d_trim + r0, nullptr, ctx->s_comp, len + r0))
+                return rc;
+    }
     if (ne)
         // every buffer's ETag in one batch: message b = its segment of the raw MD5 table (blob_utils.py:216-219)
         if (int rc = enqueue_device_batch(ctx, d_md5, d_tab + 2 * rows, d_tab + 2 * rows + ne, ne, B200H_MD5, nullptr,

@@ -111,6 +111,7 @@ struct Columns {
 
 struct Share {
     std::vector<uint64_t> idx, off, len, file_of;
+    std::vector<uint64_t> piece_of{0}, psrc, plen;  // gathered rows of a device-segments share (b200h::GatherRows)
     uint64_t bytes = 0, staged = 0;
     double ms = 0.0;
     int rc = 0;
@@ -304,9 +305,10 @@ void run_share(b200h_group* g, int j, const uint8_t* base, const char* const* pa
         for (int k = 0; k < 3; ++k)
             if (c.out[k] && c.on_device[k]) to[k] = m.share.p + col_at[k];
     }
+    const b200h::GatherRows gr{s.piece_of.data(), s.psrc.data(), s.plen.data(), b200h::gather_cap()};
     if (device_rows)
         s.rc = b200h::hash_device_rows(m.ctx, s.off.data(), s.len.data(), rows, flags, to[0], to[1], (uint64_t*)to[2],
-                                       nullptr, 0, nullptr);
+                                       nullptr, 0, nullptr, s.psrc.empty() ? nullptr : &gr);
     else
         s.rc = b200h::hash_share(m.ctx, base, s.off.data(), s.len.data(), rows, flags, to[0], to[1], (uint64_t*)to[2],
                                  paths, paths ? s.file_of.data() : nullptr, &s.staged);
@@ -338,10 +340,10 @@ void record_split(b200h_group* g, const std::vector<Share>& shares) {
 }
 
 // Deal messages (off, len, file_of) over the members (owner[i] = member of message i), run every non-empty share on
-// its member's worker, wait for all of them.
+// its member's worker, wait for all of them.  gather: the pieces of device rows that are gathered before hashing.
 int run_split(b200h_group* g, const uint8_t* base, const char* const* paths, const uint64_t* off, const uint64_t* len,
               const uint64_t* file_of, uint64_t n, uint32_t flags, const Columns& c, const uint32_t* owner,
-              bool device_rows = false) {
+              bool device_rows = false, const b200h::SegmentRows* gather = nullptr) {
     const int nm = (int)g->members.size();
     std::vector<Share> shares(nm);
     for (uint64_t i = 0; i < n; ++i) {
@@ -350,6 +352,13 @@ int run_split(b200h_group* g, const uint8_t* base, const char* const* paths, con
         s.off.push_back(off[i]);
         s.len.push_back(len[i]);
         if (file_of) s.file_of.push_back(file_of[i]);
+        if (gather) {
+            for (uint64_t p = gather->piece_of[i]; p < gather->piece_of[i + 1]; ++p) {
+                s.psrc.push_back(gather->psrc[p]);
+                s.plen.push_back(gather->plen[p]);
+            }
+            s.piece_of.push_back(s.psrc.size());
+        }
         s.bytes += len[i];
     }
     std::mutex dm;
@@ -409,6 +418,79 @@ int deliver_raw(b200h_group* g, const uint8_t* raw, uint64_t nbytes, uint8_t* ou
     const cudaError_t e = cudaMemcpy(out, raw, nbytes, cudaMemcpyDefault);
     if (e != cudaSuccess) return group_fail(g, B200H_E_CUDA, cuda_msg("cudaMemcpy (group outputs)", e));
     return 0;
+}
+
+// The group batch of device-resident rows (b200h_group_hash_device_parts / _segments): file b's rows
+// [row_of[b], row_of[b + 1]) are on device buf_dev[b]; the rows on device d are dealt over the members on d.  gather
+// (may be NULL): the pieces of the rows that must be gathered first.  one_member(ctx) = the whole call on one member.
+template <typename F>
+int group_device_rows(b200h_group* g, const std::vector<int>& buf_dev, uint64_t n, const std::vector<uint64_t>& addr,
+                      const std::vector<uint64_t>& len, const std::vector<uint64_t>& row_of, const b200h::SegmentRows* gather,
+                      uint32_t flags, uint8_t* sha256_out, uint8_t* md5_out, uint64_t* trimmed_len_out,
+                      uint8_t* etag_md5_out, F one_member) {
+    const int nm = (int)g->members.size();
+    const uint64_t rows = addr.size();
+    // the parts resident on device d are dealt over the members on d by the rule of every other group batch
+    std::vector<uint32_t> owner(rows);
+    std::vector<int> used;
+    std::vector<int> devs(buf_dev.begin(), buf_dev.end());
+    std::sort(devs.begin(), devs.end());
+    devs.erase(std::unique(devs.begin(), devs.end()), devs.end());
+    for (int d : devs) {
+        std::vector<uint64_t> idx, dlen;
+        for (uint64_t b = 0; b < n; ++b)
+            if (buf_dev[b] == d)
+                for (uint64_t r = row_of[b]; r < row_of[b + 1]; ++r) {
+                    idx.push_back(r);
+                    dlen.push_back(len[r]);
+                }
+        if (idx.empty()) continue;
+        std::vector<int> on_d;
+        for (int j = 0; j < nm; ++j)
+            if (g->members[j]->device == d) on_d.push_back(j);
+        std::vector<uint32_t> local(idx.size());
+        const int k = split_owner(dlen.data(), idx.size(), (int)on_d.size(), g->min_share, local.data());
+        for (size_t p = 0; p < idx.size(); ++p) owner[idx[p]] = (uint32_t)on_d[local[p]];
+        for (int q = 0; q < k; ++q) used.push_back(on_d[q]);
+    }
+    if (used.size() <= 1) return run_home(g, rows, len.data(), one_member, used.empty() ? 0 : used[0]);
+    const uint32_t wide = (flags & B200H_HEX_OUT) ? 2 : 1;
+    Columns c;
+    if (!etag_md5_out) {
+        c.out[0] = (flags & B200H_SHA256) ? sha256_out : nullptr;
+        c.out[1] = (flags & B200H_MD5) ? md5_out : nullptr;
+        c.out[2] = (uint8_t*)trimmed_len_out;
+        c.width[0] = 32 * wide;
+        c.width[1] = 16 * wide;
+        if (int rc = classify_outputs(g, c)) return rc;
+        return run_split(g, nullptr, nullptr, addr.data(), len.data(), nullptr, rows, flags, c, owner.data(), true, gather);
+    }
+    // ETags need every raw MD5 row in one place: the shares land in host tables, the ETags are one batch over
+    // segments of the MD5 table on the home member, then the columns go where the caller wants them.
+    std::vector<uint8_t> tsha((flags & B200H_SHA256) ? rows * 32 : 0), tmd5(rows * 16 + 16);
+    std::vector<uint64_t> ttrim(rows);
+    c.out[0] = tsha.empty() ? nullptr : tsha.data();
+    c.out[1] = tmd5.data();
+    c.out[2] = (uint8_t*)ttrim.data();
+    c.width[0] = 32;
+    c.width[1] = 16;
+    if (int rc = run_split(g, nullptr, nullptr, addr.data(), len.data(), nullptr, rows, flags & ~B200H_HEX_OUT, c,
+                           owner.data(), true, gather))
+        return rc;
+    std::vector<uint64_t> eoff(n), elen(n);
+    for (uint64_t b = 0; b < n; ++b) {
+        eoff[b] = 16 * row_of[b];
+        elen[b] = 16 * (row_of[b + 1] - row_of[b]);
+    }
+    b200h_ctx* home = g->members[0]->ctx;
+    uint64_t staged = 0;
+    if (int rc = b200h::hash_share(home, tmd5.data(), eoff.data(), elen.data(), n, B200H_MD5, nullptr, etag_md5_out,
+                                   nullptr, nullptr, nullptr, &staged))
+        return group_fail(g, rc, member_prefix(g, 0) + b200h_last_error(home));
+    const bool hex = (flags & B200H_HEX_OUT) != 0;
+    if (int rc = deliver_raw(g, tsha.data(), tsha.size(), sha256_out, hex)) return rc;
+    if (int rc = deliver_raw(g, tmd5.data(), rows * 16, md5_out, hex)) return rc;
+    return deliver_raw(g, (const uint8_t*)ttrim.data(), rows * 8, (uint8_t*)trimmed_len_out, false);
 }
 
 }  // namespace
@@ -555,75 +637,43 @@ int b200h_group_hash_device_parts(b200h_group* g, const void* const* d_bufs, con
     }
     std::vector<uint64_t> addr, len, row_of;
     b200h::device_part_rows(d_bufs, sizes, n, part_len, addr, len, row_of);
-    const uint64_t rows = addr.size();
-    // the parts resident on device d are dealt over the members on d by the rule of every other group batch
-    std::vector<uint32_t> owner(rows);
-    std::vector<int> used;
-    std::vector<int> devs(buf_dev.begin(), buf_dev.end());
-    std::sort(devs.begin(), devs.end());
-    devs.erase(std::unique(devs.begin(), devs.end()), devs.end());
-    for (int d : devs) {
-        std::vector<uint64_t> idx, dlen;
-        for (uint64_t b = 0; b < n; ++b)
-            if (buf_dev[b] == d)
-                for (uint64_t r = row_of[b]; r < row_of[b + 1]; ++r) {
-                    idx.push_back(r);
-                    dlen.push_back(len[r]);
-                }
-        if (idx.empty()) continue;
-        std::vector<int> on_d;
-        for (int j = 0; j < nm; ++j)
-            if (g->members[j]->device == d) on_d.push_back(j);
-        std::vector<uint32_t> local(idx.size());
-        const int k = split_owner(dlen.data(), idx.size(), (int)on_d.size(), g->min_share, local.data());
-        for (size_t p = 0; p < idx.size(); ++p) owner[idx[p]] = (uint32_t)on_d[local[p]];
-        for (int q = 0; q < k; ++q) used.push_back(on_d[q]);
+    return group_device_rows(g, buf_dev, n, addr, len, row_of, nullptr, flags, sha256_out, md5_out, trimmed_len_out,
+                             etag_md5_out, [&](b200h_ctx* m) {
+                                 return b200h_hash_device_parts(m, d_bufs, sizes, n, part_len, flags, sha256_out, md5_out,
+                                                                trimmed_len_out, etag_md5_out);
+                             });
+}
+
+int b200h_group_hash_device_segments(b200h_group* g, const void* const* d_segs, const uint64_t* seg_sizes,
+                                     const uint64_t* seg_of, uint64_t n_files, uint64_t part_len, uint32_t flags,
+                                     uint8_t* sha256_out, uint8_t* md5_out, uint64_t* trimmed_len_out,
+                                     uint8_t* etag_md5_out) {
+    if (!g) return B200H_E_INVALID;
+    const std::string bad = b200h::segment_args_error(d_segs, seg_sizes, seg_of, n_files);
+    if (!bad.empty()) return group_fail(g, B200H_E_INVALID, bad);
+    if (!(flags & (B200H_SHA256 | B200H_MD5))) return group_fail(g, B200H_E_INVALID, "flags select neither SHA256 nor MD5");
+    if (etag_md5_out && !(flags & B200H_MD5)) return group_fail(g, B200H_E_INVALID, "etag requires B200H_MD5");
+    const int nm = (int)g->members.size();
+    // where every file lives; a file may only be hashed by the members on its device
+    std::vector<int> file_dev;
+    std::string err;
+    if (b200h::segment_devices(d_segs, seg_sizes, seg_of, n_files, file_dev, &err)) return group_fail(g, B200H_E_INVALID, err);
+    for (uint64_t i = 0; i < n_files; ++i) {
+        const int d = file_dev[i];
+        bool covered = d < 0;
+        for (int j = 0; j < nm && !covered; ++j) covered = g->members[j]->device == d;
+        if (!covered)
+            return group_fail(g, B200H_E_INVALID, "file " + std::to_string(i) + " is on cuda:" + std::to_string(d) +
+                                                      ", which is not in the group");
+        if (d < 0) file_dev[i] = g->members[0]->device;  // an empty file reads nothing: the home device takes it
     }
-    if (used.size() <= 1)
-        return run_home(
-            g, rows, len.data(),
-            [&](b200h_ctx* m) {
-                return b200h_hash_device_parts(m, d_bufs, sizes, n, part_len, flags, sha256_out, md5_out, trimmed_len_out,
-                                               etag_md5_out);
-            },
-            used.empty() ? 0 : used[0]);
-    const uint32_t wide = (flags & B200H_HEX_OUT) ? 2 : 1;
-    Columns c;
-    if (!etag_md5_out) {
-        c.out[0] = (flags & B200H_SHA256) ? sha256_out : nullptr;
-        c.out[1] = (flags & B200H_MD5) ? md5_out : nullptr;
-        c.out[2] = (uint8_t*)trimmed_len_out;
-        c.width[0] = 32 * wide;
-        c.width[1] = 16 * wide;
-        if (int rc = classify_outputs(g, c)) return rc;
-        return run_split(g, nullptr, nullptr, addr.data(), len.data(), nullptr, rows, flags, c, owner.data(), true);
-    }
-    // ETags need every raw MD5 row in one place: the shares land in host tables, the ETags are one batch over
-    // segments of the MD5 table on the home member, then the columns go where the caller wants them.
-    std::vector<uint8_t> tsha((flags & B200H_SHA256) ? rows * 32 : 0), tmd5(rows * 16 + 16);
-    std::vector<uint64_t> ttrim(rows);
-    c.out[0] = tsha.empty() ? nullptr : tsha.data();
-    c.out[1] = tmd5.data();
-    c.out[2] = (uint8_t*)ttrim.data();
-    c.width[0] = 32;
-    c.width[1] = 16;
-    if (int rc = run_split(g, nullptr, nullptr, addr.data(), len.data(), nullptr, rows, flags & ~B200H_HEX_OUT, c,
-                           owner.data(), true))
-        return rc;
-    std::vector<uint64_t> eoff(n), elen(n);
-    for (uint64_t b = 0; b < n; ++b) {
-        eoff[b] = 16 * row_of[b];
-        elen[b] = 16 * (row_of[b + 1] - row_of[b]);
-    }
-    b200h_ctx* home = g->members[0]->ctx;
-    uint64_t staged = 0;
-    if (int rc = b200h::hash_share(home, tmd5.data(), eoff.data(), elen.data(), n, B200H_MD5, nullptr, etag_md5_out,
-                                   nullptr, nullptr, nullptr, &staged))
-        return group_fail(g, rc, member_prefix(g, 0) + b200h_last_error(home));
-    const bool hex = (flags & B200H_HEX_OUT) != 0;
-    if (int rc = deliver_raw(g, tsha.data(), tsha.size(), sha256_out, hex)) return rc;
-    if (int rc = deliver_raw(g, tmd5.data(), rows * 16, md5_out, hex)) return rc;
-    return deliver_raw(g, (const uint8_t*)ttrim.data(), rows * 8, (uint8_t*)trimmed_len_out, false);
+    b200h::SegmentRows sr;
+    b200h::segment_rows(d_segs, seg_sizes, seg_of, n_files, part_len, sr);
+    return group_device_rows(g, file_dev, n_files, sr.addr, sr.len, sr.row_of, &sr, flags, sha256_out, md5_out,
+                             trimmed_len_out, etag_md5_out, [&](b200h_ctx* m) {
+                                 return b200h_hash_device_segments(m, d_segs, seg_sizes, seg_of, n_files, part_len, flags,
+                                                                   sha256_out, md5_out, trimmed_len_out, etag_md5_out);
+                             });
 }
 
 int b200h_group_last_split(b200h_group* g, uint64_t* messages_out, uint64_t* bytes_out, uint64_t* staged_bytes_out,
